@@ -375,6 +375,21 @@ def pin_to_gpu_cpus(index):
     return None
 
 
+STEP_COUNTS = ("plies", "sequences", "games_finished", "p1_wins", "truncated")
+
+
+def dump_outputs(out_dir, eng, stats):
+    """What the last timed step hands its caller, as .npy files for comparing two builds output for output: the
+    population after it (records int8[G,32] -> records.npy float32; ply numbers and game ids -> float64) and the step's
+    game counters in STEP_COUNTS order (step_counts.npy float64).  9 MB for one GPU's 65,536 games (rank 0's)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rec, ply, gid = eng.selfplay_read()
+    for name, a in (("records", rec.astype(np.float32)), ("ply", ply.astype(np.float64)), ("game_id", gid.astype(np.float64)),
+                    ("step_counts", np.array([stats[k] for k in STEP_COUNTS], np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -429,6 +444,8 @@ def run_ours(args):
     barrier()
     wall = time.perf_counter() - t_wall0
     launches = eng.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, st)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     counts = torch.tensor([plies, seqs, scored], dtype=torch.float64, device=dev)
@@ -744,7 +761,11 @@ def main():
     ap.add_argument("--no-td-parity", action="store_true", help="skip the TD parity block of the td_round object")
     ap.add_argument("--td-games", type=int, default=-1,
                     help="games per GPU in the TD(lambda) round leg (0 = skip; default: 262,144 on one GPU, 2^20 / N on N)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed self-play step computed to DIR/<name>.npy (population and game counters)")
     args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs --steps >= 1: it writes what the last timed step computed")
     if args.impl == "reference":
         run_reference(args)
     else:

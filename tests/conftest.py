@@ -37,15 +37,6 @@ def orc():
     return Oracle()
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """The unmodified reference engine, if oracle/_ref was built (it is, wherever /root/reference was visible)."""
-    from oracle.oracle import RefHarness
-    if not RefHarness.available():
-        pytest.skip("oracle/_ref/libref_harness.so not built (no /root/reference on this box)")
-    return RefHarness()
-
-
 def load_golden(name):
     """Fixture file as a plain dict (NpzFile re-reads the archive on every [] access)."""
     with np.load(os.path.join(GOLDEN, name), allow_pickle=False) as z:

@@ -260,11 +260,22 @@ def test_greedy_games_golden(orc, golden):
         assert soft <= max(2, len(pre) // 10), (name, soft)
 
 
-# ------------------------------------------------------------------ live reference, fresh seeds
+# ------------------------------------------------------------------ reference on fresh seeds (recorded; live where built)
 
-def test_fuzz_against_live_reference(orc, ref):
+def test_fuzz_against_reference(orc, golden):
+    """4,000 fresh seeded positions: sequence count and ordered digest against the reference's, recorded in
+    tests/golden/fuzz_summary.npz (provenance: tests/golden/make_recorded.py), and, where oracle/_ref holds the reference
+    engine, every ordered sequence list against it live."""
     from bgx.synth import make_queries
+    from oracle.oracle import RefHarness
     q, _ = make_queries(4000, seed=987654)
+    g = golden("fuzz_summary.npz")
+    assert np.array_equal(q, g["queries"])
+    n, _, d = orc.turn_summary_batch(q)
+    assert np.array_equal(n, g["n_seq"]) and np.array_equal(d, g["digest"])
+    if not RefHarness.available():
+        return
+    ref = RefHarness()
     for r in q:
         s = r[:28].astype(np.int32)
         a = orc.turn_sequences(s, r[28], r[29], r[30])
