@@ -219,6 +219,38 @@ class BatchEngine:
                                            L.ptr(chosen), L.ptr(moves), L.ptr(moves_len), L.ptr(value),
                                            L.ptr(n_seq), L.ptr(n_scored)))
 
+    def select_moves_2ply_host(self, queries, max_candidates=0, out=None):
+        """Two-ply move selection (bgx_select_moves_2ply): every distinct afterstate, or the `max_candidates` best by one-ply
+        value, valued by the expectation over the opponent's 21 rolls of the opponent's greedy reply.
+        -> dict(chosen int8[n,32], moves int8[n,4,2], moves_len int8[n], value f32[n], n_candidates int32[n], n_expanded int32[n])"""
+        q = _records(queries)
+        n = q.shape[0]
+        o = out or {}
+        o.setdefault("chosen", np.zeros((n, 32), np.int8))
+        o.setdefault("moves", np.zeros((n, 4, 2), np.int8))
+        o.setdefault("moves_len", np.zeros(n, np.int8))
+        o.setdefault("value", np.zeros(n, np.float32))
+        o.setdefault("n_candidates", np.zeros(n, np.int32))
+        o.setdefault("n_expanded", np.zeros(n, np.int32))
+        L.check(self._lib.bgx_select_moves_2ply_host(self._h, q.ctypes.data, n, int(max_candidates),
+                                                     L.ptr(o["chosen"]), L.ptr(o["moves"]), L.ptr(o["moves_len"]),
+                                                     L.ptr(o["value"]), L.ptr(o["n_candidates"]), L.ptr(o["n_expanded"])))
+        return o
+
+    def select_moves_2ply(self, queries, max_candidates=0, chosen=None, moves=None, moves_len=None, value=None,
+                          n_candidates=None, n_expanded=None):
+        """select_moves_2ply_host on device tensors (the engine's stream)"""
+        L.check(self._lib.bgx_select_moves_2ply(self._h, L.ptr(queries), queries.shape[0], int(max_candidates),
+                                                L.ptr(chosen), L.ptr(moves), L.ptr(moves_len), L.ptr(value),
+                                                L.ptr(n_candidates), L.ptr(n_expanded)))
+
+    def twoply_stage_ms(self):
+        """Stage times (ms) of the two-ply calls made since the last read with set_option("twoply_timing", 1):
+        candidates, expand, replies, reduce"""
+        ms = np.zeros(4, np.float64)
+        L.check(self._lib.bgx_twoply_stage_ms(self._h, ms.ctypes.data))
+        return dict(zip(("candidates", "expand", "replies", "reduce"), ms.tolist()))
+
     # ------------------------------------------------------------------ self-play population
     def selfplay_init(self, n_slots, first_id=0, id_stride=None, seed=0x5EED2026, first_mover=L.FIRST_ROLLOFF,
                       traj_cap=0, record_chosen=False):

@@ -6,8 +6,9 @@ All games advance in lockstep, one ply per iteration: the games whose mover is p
 go through one `bgx_select_moves` launch of engine A, the others through engine B, then `bgx_advance`
 checks for the end of the game, flips the mover and rolls the next dice (Philox, the self-play dice
 rule, so every game can be replayed into the reference through `Game.setDice`).  A policy is a
-weight tuple (greedy, epsilon = 0: `make_move`) or the string "random" (`_random_move`,
-benchmark.py:54-61: a uniformly random legal sequence).
+weight tuple (greedy, epsilon = 0: `make_move`), the string "random" (`_random_move`,
+benchmark.py:54-61: a uniformly random legal sequence) or a `TwoPly` (the same net looking one roll
+ahead: `bgx_select_moves_2ply`).
 """
 import numpy as np
 import torch
@@ -16,6 +17,17 @@ from .engine import BatchEngine
 from .synth import START_BOARD
 
 RANDOM = "random"
+
+
+class TwoPly:
+    """Two-ply policy: `weights` looking one roll ahead (BatchEngine.select_moves_2ply); `candidates` = how many of the best
+    one-ply afterstates are expanded (0 = all of them)."""
+
+    def __init__(self, weights, candidates=0):
+        if int(candidates) < 0:
+            raise ValueError("candidates must be >= 0")
+        self.weights = weights
+        self.candidates = int(candidates)
 
 
 class Arena:
@@ -34,6 +46,10 @@ class Arena:
             e.close()
 
     def _load(self, k, policy):
+        """-> (epsilon, two-ply candidates or None) of the policy now loaded into engine k"""
+        if isinstance(policy, TwoPly):
+            self.eng[k].set_weights(*policy.weights)
+            return 0.0, policy.candidates
         if isinstance(policy, str):
             if policy != RANDOM:
                 raise ValueError(policy)
@@ -41,9 +57,9 @@ class Arena:
                 self._dummy = (np.zeros((128, 198), np.float32), np.zeros(128, np.float32),
                                np.zeros((1, 128), np.float32), np.zeros(1, np.float32))
             self.eng[k].set_weights(*self._dummy)       # the random policy never evaluates
-            return 1.0
+            return 1.0, None
         self.eng[k].set_weights(*policy)
-        return 0.0
+        return 0.0, None
 
     def play(self, policy_a, policy_b, side_of_a, first_mover, seed=0x5EED2026, max_plies=4096, record=False):
         """n games; game i: policy A plays PLAYER `side_of_a[i]` (0/1), PLAYER `first_mover[i]` moves first.
@@ -51,7 +67,8 @@ class Arena:
         dev = self.device
         side = torch.as_tensor(np.asarray(side_of_a), dtype=torch.int8, device=dev)
         n = side.numel()
-        eps = [self._load(0, policy_a), self._load(1, policy_b)]
+        (eps_a, two_a), (eps_b, two_b) = self._load(0, policy_a), self._load(1, policy_b)
+        eps, two = [eps_a, eps_b], [two_a, two_b]
         start = np.zeros((n, 32), np.int8)
         start[:, :24] = START_BOARD
         start[:, 28] = np.asarray(first_mover, np.int8) ^ 1           # bgx_advance flips it and rolls ply 0
@@ -73,7 +90,10 @@ class Arena:
                     continue
                 q = rec[idx].contiguous()
                 ch = torch.empty_like(q)
-                self.eng[k].select_moves(q, epsilon=eps[k], seed=(seed ^ ((ply + 1) << 32)) & (2 ** 64 - 1), chosen=ch)
+                if two[k] is not None:
+                    self.eng[k].select_moves_2ply(q, two[k], chosen=ch)
+                else:
+                    self.eng[k].select_moves(q, epsilon=eps[k], seed=(seed ^ ((ply + 1) << 32)) & (2 ** 64 - 1), chosen=ch)
                 w = torch.empty(m, dtype=torch.int8, device=dev)
                 nxt = torch.empty_like(q)
                 self.eng[k].advance(ch, nxt, seed, ply + 1, idx, w)

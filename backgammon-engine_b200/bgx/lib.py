@@ -63,6 +63,8 @@ _SIGNATURES = {
     "bgx_evaluate_host": (C.c_int, [_vp, _vp, _i64, _vp]),
     "bgx_select_moves": (C.c_int, [_vp, _vp, _i64, C.c_float, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_select_moves_host": (C.c_int, [_vp, _vp, _i64, C.c_float, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "bgx_select_moves_2ply": (C.c_int, [_vp, _vp, _i64, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "bgx_select_moves_2ply_host": (C.c_int, [_vp, _vp, _i64, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_select_moves_host_async": (C.c_int, [_vp, C.c_int, _vp, _i64, C.c_float, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_play_ply_host_async": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _i64, C.c_float, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
     "bgx_play_ply_restart_host_async": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _i64, C.c_int, _i64, C.c_float, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
@@ -97,6 +99,7 @@ _SIGNATURES = {
     "bgx_kernel_config": (C.c_int, [_vp, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "bgx_sfu_monotone": (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
     "bgx_set_option": (C.c_int, [_vp, C.c_char_p, _i64]),
+    "bgx_twoply_stage_ms": (C.c_int, [_vp, _vp]),
     "bgx_td_profile": (C.c_int, [_vp, C.c_int, _vp]),
     "bgx_device_props": (C.c_int, [_vp, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_i64)]),
 }

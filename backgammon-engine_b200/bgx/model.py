@@ -9,7 +9,7 @@ names and shapes (state_dict compatible with models/*.pth), `learning_rate`, `la
 `make_move`, `initialize_traces`, `initialize_weights`.
 
 Added: `engine()` (a BatchEngine holding these weights), `make_moves_batch` (batched
-make_move over many games at once) — the per-object `make_move` stays a host-side loop because
+make_move over many games at once, greedy or two-ply) — the per-object `make_move` stays a host-side loop because
 one position per call cannot amortise a kernel launch; the batch calls are the fast path.
 """
 import random
@@ -173,9 +173,15 @@ class TDLGammonModel(nn.Module):
         self.load_weights_from(self._engine)
         self._uploaded = self._weights_version()
 
-    def make_moves_batch(self, games, epsilon=0.0, seed=0, device=0):
+    def make_moves_batch(self, games, epsilon=0.0, seed=0, device=0, plies=1, candidates=0):
         """make_move for a list of compat Game objects in ONE kernel launch; applies the chosen
-        sequences to the games and returns them (list[list[tuple]])."""
+        sequences to the games and returns them (list[list[tuple]]).  plies=2 looks one roll ahead
+        (BatchEngine.select_moves_2ply_host; `candidates` = how many of the best one-ply afterstates
+        are expanded, 0 = all); it has no exploration, so epsilon must be 0 there."""
+        if plies not in (1, 2):
+            raise ValueError(f"plies must be 1 or 2, not {plies}")
+        if plies == 2 and epsilon > 0.0:
+            raise ValueError("two-ply move selection has no epsilon exploration")
         q = np.zeros((len(games), 32), np.int8)
         for i, g in enumerate(games):
             q[i, :24] = g.getGameBoard()
@@ -183,7 +189,10 @@ class TDLGammonModel(nn.Module):
             q[i, 26], q[i, 27] = g.getBornOffCount(0), g.getBornOffCount(1)
             q[i, 28] = g.getTurn()
             q[i, 29:31] = g.get_last_dice()
-        out = self.engine(device).select_moves_host(q, epsilon=epsilon, seed=seed)
+        if plies == 2:
+            out = self.engine(device).select_moves_2ply_host(q, max_candidates=candidates)
+        else:
+            out = self.engine(device).select_moves_host(q, epsilon=epsilon, seed=seed)
         result = []
         for i, g in enumerate(games):
             seq = [(int(o), int(d)) for o, d in out["moves"][i, : out["moves_len"][i]]]

@@ -274,6 +274,21 @@ class BatchEngine {
         d["chosen"] = chosen; d["moves"] = moves; d["moves_len"] = len; d["value"] = value; d["n_seq"] = n_seq; d["n_scored"] = n_scored;
         return d;
     }
+    py::dict make_moves_2ply(I8 q, int32_t max_candidates)
+    {
+        int64_t n = rows(q);
+        py::array_t<int8_t> chosen({(py::ssize_t)n, (py::ssize_t)32}), moves({(py::ssize_t)n, (py::ssize_t)4, (py::ssize_t)2}), len(n);
+        py::array_t<float> value(n);
+        py::array_t<int32_t> n_cand(n), n_exp(n);
+        {
+            py::gil_scoped_release nogil;
+            Game::check(bgx_select_moves_2ply_host(e_, q.data(), n, max_candidates, chosen.mutable_data(), moves.mutable_data(),
+                                                   len.mutable_data(), value.mutable_data(), n_cand.mutable_data(), n_exp.mutable_data()));
+        }
+        py::dict d;
+        d["chosen"] = chosen; d["moves"] = moves; d["moves_len"] = len; d["value"] = value; d["n_candidates"] = n_cand; d["n_expanded"] = n_exp;
+        return d;
+    }
     py::array_t<float> encode(I8 q)
     {
         int64_t n = rows(q);
@@ -440,6 +455,7 @@ PYBIND11_MODULE(backgammon_env, m)
         .def("set_weights", &BatchEngine::set_weights)
         .def("evaluate_turn_sequences_summary", &BatchEngine::evaluate_turn_sequences_summary)
         .def("make_moves", &BatchEngine::make_moves, py::arg("queries"), py::arg("epsilon") = 0.0f, py::arg("seed") = 0)
+        .def("make_moves_2ply", &BatchEngine::make_moves_2ply, py::arg("queries"), py::arg("max_candidates") = 0)
         .def("encode", &BatchEngine::encode)
         .def("evaluate", &BatchEngine::evaluate)
         .def("get_weights", &BatchEngine::get_weights)

@@ -5,6 +5,7 @@
 #include "bgx_internal.h"
 #include "bgx_kernels.cuh"
 #include "bgx_td.cuh"
+#include "bgx_twoply.cuh"
 
 #include <dlfcn.h>
 
@@ -44,8 +45,8 @@ struct bgx_engine {
     int32_t *fixed = nullptr;     // [198][128] W1 transposed in fixed point (ply kernels, k_evaluate)
     float *aux = nullptr;         // [4] derived scalars: [0] fixed-point scale S, [1] 1/S
     bool have_weights = false;
-    // scratch
-    static constexpr int kScratch = 12;
+    // scratch ([12..] belong to the two-ply path)
+    static constexpr int kScratch = 32;
     void *dbuf[kScratch] = {};
     size_t dcap[kScratch] = {};
     unsigned long long *counter = nullptr;   // work queue
@@ -77,6 +78,10 @@ struct bgx_engine {
     long long select_order_max = 1 << 21;    // launches up to this many queries get a sorted queue (64 B of scratch per query)
     int select_urgent_min = 7, select_giant_min = kGiantMinChildren, select_urgent_from_pct = 0;   // k_select help policy
     int selfplay_warps = 20, select_warps = 20;   // warps per CTA of k_selfplay / k_select (measured best: 96 registers, 86 cache sets per warp)
+    long long twoply_chunk = 0;              // replies per k_select launch of a two-ply call (0: kTwoplyChunk)
+    bool twoply_timing = false;              // time the stages of a two-ply call (synchronises between them)
+    double twoply_ms[4] = {};                // candidates, expand, replies, reduce: accumulated stage times
+    cudaEvent_t tp0 = nullptr, tp1 = nullptr;
     // bookkeeping
     long long launches = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_sync = nullptr;
@@ -166,6 +171,8 @@ static int create_into(bgx_engine *e, int device, const cudaDeviceProp &prop)
     CU(cudaEventCreateWithFlags(&e->ev_sync, cudaEventDisableTiming));
     CU(cudaFuncSetAttribute(k_evaluate, cudaFuncAttributeMaxDynamicSharedMemorySize, kEvalSmem));
     CU(cudaFuncSetAttribute(k_encode, cudaFuncAttributeMaxDynamicSharedMemorySize, kEncSmem));
+    CU(cudaFuncSetAttribute(k_candidates, cudaFuncAttributeMaxDynamicSharedMemorySize, kEvalSmem));
+    CU(cudaFuncSetAttribute(k_twoply_reduce, cudaFuncAttributeMaxDynamicSharedMemorySize, kEvalSmem));
     e->lane_grid = e->sm_count / 2;
     static_assert(ply_smem<16, 109>() <= 232448 && ply_smem<20, 86>() <= 232448 && ply_smem<24, 72>() <= 232448 && ply_smem<32, 53>() <= 232448,
                   "fused ply kernels: shared memory per CTA");
@@ -231,6 +238,10 @@ int bgx_set_option(bgx_engine *e, const char *key, int64_t value)
     else if (k == "select_urgent_min") e->select_urgent_min = (int)value;
     else if (k == "select_giant_min") e->select_giant_min = (int)value;
     else if (k == "select_urgent_from_pct") e->select_urgent_from_pct = (int)value;
+    else if (k == "twoply_chunk") {
+        if (value < 0) { set_error("bgx_set_option: twoply_chunk must be >= 0"); return BGX_E_INVALID; }
+        e->twoply_chunk = (long long)value;
+    } else if (k == "twoply_timing") e->twoply_timing = value != 0;
     else { set_error("bgx_set_option: unknown option '%s'", key); return BGX_E_INVALID; }
     return BGX_OK;
 }
@@ -247,6 +258,8 @@ int bgx_destroy(bgx_engine *e)
     if (e->ev0) cudaEventDestroy(e->ev0);
     if (e->ev1) cudaEventDestroy(e->ev1);
     if (e->ev_sync) cudaEventDestroy(e->ev_sync);
+    if (e->tp0) cudaEventDestroy(e->tp0);
+    if (e->tp1) cudaEventDestroy(e->tp1);
     for (bgx_lane &l : e->lanes) {
         if (l.stream) cudaStreamDestroy(l.stream);
         if (l.done) cudaEventDestroy(l.done);
@@ -609,6 +622,196 @@ int bgx_select_moves_host(bgx_engine *e, const int8_t *queries, int64_t n, float
     if (n_seq) CU(cudaMemcpyAsync(n_seq, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
     if (n_scored) CU(cudaMemcpyAsync(n_scored, ds, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
+    return BGX_OK;
+}
+
+// ------------------------------------------------------------------------ two-ply move selection (DESIGN 7c)
+
+constexpr long long kTwoplyChunk = 1ll << 21;   // replies per k_select launch: the sorted-queue limit (select_order_max default)
+
+// with "twoply_timing": the time since the previous mark goes to stage k (0 candidates, 1 expand, 2 replies, 3 reduce)
+static int twoply_mark(bgx_engine *e, int k)
+{
+    if (!e->twoply_timing) return BGX_OK;
+    CU(cudaEventRecord(e->tp1, e->stream));
+    CU(cudaEventSynchronize(e->tp1));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, e->tp0, e->tp1));
+    e->twoply_ms[k] += ms;
+    CU(cudaEventRecord(e->tp0, e->stream));
+    return BGX_OK;
+}
+#define TWOPLY_MARK(e, k) do { const int rc__ = twoply_mark(e, k); if (rc__ != BGX_OK) return rc__; } while (0)
+
+// exclusive prefix sum of cnt[n] into offsets[n + 1] (the k_scan_* launches of bgx_enumerate_count)
+static int scan_counts(bgx_engine *e, const int32_t *cnt, int64_t n, long long *offsets, long long *sums)
+{
+    const int n_tiles = (int)((n + kScanTile - 1) / kScanTile);
+    k_scan_tiles<<<n_tiles, kScanThreads, 0, e->stream>>>(cnt, n, offsets, sums);
+    k_scan_sums<<<1, 1024, 0, e->stream>>>(sums, n_tiles);
+    k_scan_add<<<(unsigned)((n + kScanThreads - 1) / kScanThreads), kScanThreads, 0, e->stream>>>(offsets, n, sums, n_tiles);
+    e->launches += 3;
+    CU(cudaGetLastError());
+    return BGX_OK;
+}
+
+int bgx_select_moves_2ply(bgx_engine *e, const int8_t *queries, int64_t n, int32_t max_candidates,
+                          int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value, int32_t *n_candidates, int32_t *n_expanded)
+{
+    USE(e);
+    NEED(queries && n >= 0 && max_candidates >= 0, "bad argument");
+    if (!e->have_weights) { set_error("bgx_select_moves_2ply: weights not set"); return BGX_E_STATE; }
+    if (n == 0) return BGX_OK;
+    int rc = ensure_uniq_tables(e);
+    if (rc) return rc;
+    if (e->twoply_timing) {
+        if (!e->tp0) { CU(cudaEventCreate(&e->tp0)); CU(cudaEventCreate(&e->tp1)); }
+        CU(cudaEventRecord(e->tp0, e->stream));
+    }
+    const int n_tiles = (int)((n + kScanTile - 1) / kScanTile);
+    void *d_nseq, *d_u, *d_dig, *d_cnt, *d_off, *d_sums, *d_flags, *d_nexp, *d_eoff;
+    if ((rc = scratch(e, 12, (size_t)n * 4, &d_nseq))) return rc;
+    if ((rc = scratch(e, 13, (size_t)n * 4, &d_u))) return rc;
+    if ((rc = scratch(e, 14, (size_t)n * 8, &d_dig))) return rc;
+    if ((rc = scratch(e, 15, (size_t)n * 4, &d_cnt))) return rc;
+    if ((rc = scratch(e, 16, (size_t)(n + 1) * 8, &d_off))) return rc;
+    if ((rc = scratch(e, 17, (size_t)(n_tiles + 1) * 8, &d_sums))) return rc;
+    if ((rc = scratch(e, 18, 16, &d_flags))) return rc;
+    if ((rc = scratch(e, 19, (size_t)n * 4, &d_nexp))) return rc;
+    if ((rc = scratch(e, 20, (size_t)(n + 1) * 8, &d_eoff))) return rc;
+    int32_t *cnt = (int32_t *)d_cnt, *nexp = (int32_t *)d_nexp;
+    long long *off = (long long *)d_off, *eoff = (long long *)d_eoff, *sums = (long long *)d_sums;
+    int *flags = (int *)d_flags;
+
+    // 1. candidates: U per query (the summary walk), their offsets, then every distinct afterstate with its first sequence and V
+    CU(cudaMemsetAsync(flags, 0, 16, e->stream));
+    CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
+    k_enumerate_summary<<<e->uniq_grid, kGameThreads, 0, e->stream>>>(queries, n, (int32_t *)d_nseq, (int32_t *)d_u,
+                                                                       (unsigned long long *)d_dig, e->uniq_tables, e->uniq_gens, e->counter);
+    k_twoply_count<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>((const int32_t *)d_u, n, cnt, flags);
+    e->launches += 2;
+    if ((rc = scan_counts(e, cnt, n, off, sums))) return rc;
+    long long n_cand = 0;
+    int hflags[4] = {};
+    CU(cudaMemcpyAsync(&n_cand, off + n, 8, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaMemcpyAsync(hflags, flags, 16, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    if (hflags[0]) {
+        set_error("bgx_select_moves_2ply: a query has more distinct afterstates than the exact-dedup table holds (%d)", kUniqSlots);
+        return BGX_E_CAPACITY;
+    }
+    void *d_rec = nullptr, *d_mv = nullptr, *d_len = nullptr, *d_val = nullptr, *d_exp = nullptr, *d_e2 = nullptr;
+    const size_t C = (size_t)(n_cand > 0 ? n_cand : 1);
+    if ((rc = scratch(e, 21, C * 32, &d_rec))) return rc;
+    if ((rc = scratch(e, 22, C * 8, &d_mv))) return rc;
+    if ((rc = scratch(e, 23, C, &d_len))) return rc;
+    if ((rc = scratch(e, 24, C * 4, &d_val))) return rc;
+    if ((rc = scratch(e, 25, C, &d_exp))) return rc;
+    if ((rc = scratch(e, 26, C * 4, &d_e2))) return rc;
+    int8_t *rec = (int8_t *)d_rec, *cmv = (int8_t *)d_mv, *clen = (int8_t *)d_len, *expand = (int8_t *)d_exp;
+    float *val = (float *)d_val, *e2 = (float *)d_e2;
+    if (n_cand > 0) {
+        CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
+        k_candidates<<<game_grid(e), kGameThreads, kEvalSmem, e->stream>>>(queries, n, cnt, off, rec, cmv, clen, val, e->uniq_tables,
+                                                                           e->uniq_gens, e->counter, flags, e->fixed);
+        e->launches++;
+        CU(cudaGetLastError());
+    }
+    TWOPLY_MARK(e, 0);
+
+    // 2. which candidates are expanded, and the list of them
+    const unsigned small_grid = (unsigned)std::min<long long>((n + 7) / 8, (long long)e->sm_count * 8);
+    k_twoply_expand<<<small_grid, 256, 0, e->stream>>>(queries, n, cnt, off, rec, val, max_candidates, expand, nexp);
+    e->launches++;
+    if ((rc = scan_counts(e, nexp, n, eoff, sums))) return rc;
+    long long n_exp = 0;
+    CU(cudaMemcpyAsync(&n_exp, eoff + n, 8, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaMemcpyAsync(hflags, flags, 16, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    if (hflags[0] & 2) {
+        set_error("bgx_select_moves_2ply: the candidate walk disagreed with the summary walk");
+        return BGX_E_CUDA;
+    }
+    void *d_list = nullptr;
+    if ((rc = scratch(e, 27, (size_t)(n_exp > 0 ? n_exp : 1) * 8, &d_list))) return rc;
+    long long *list = (long long *)d_list;
+    if (n_exp > 0) {
+        k_twoply_list<<<small_grid, 256, 0, e->stream>>>(n, cnt, off, expand, eoff, list);
+        e->launches++;
+    }
+    TWOPLY_MARK(e, 1);
+
+    // 3. replies in chunks: 21 records per expanded candidate, k_select (values only), the expectation
+    const long long chunk_replies = std::max<long long>(e->twoply_chunk > 0 ? e->twoply_chunk : kTwoplyChunk, kRolls);
+    const long long per_chunk = chunk_replies / kRolls;
+    const long long cap_replies = std::min<long long>(n_exp, per_chunk) * kRolls;
+    void *d_rep = nullptr, *d_rval = nullptr, *region = nullptr;
+    if (n_exp > 0) {
+        if ((rc = scratch(e, 28, (size_t)cap_replies * 32, &d_rep))) return rc;
+        if ((rc = scratch(e, 29, (size_t)cap_replies * 4, &d_rval))) return rc;
+        if (cap_replies <= e->select_order_max && (rc = scratch(e, 30, (size_t)cap_replies * kOrderBuckets * 4, &region))) return rc;
+    }
+    for (long long e0 = 0; e0 < n_exp; e0 += per_chunk) {
+        const long long e1 = std::min(n_exp, e0 + per_chunk);
+        const long long nr = (e1 - e0) * kRolls;
+        k_twoply_replies<<<(unsigned)std::min<long long>((nr + 7) / 8, (long long)e->sm_count * 16), 256, 0, e->stream>>>(list, e0, nr, rec,
+                                                                                                                        (int8_t *)d_rep);
+        e->launches++;
+        const SelectOut out = {nullptr, nullptr, nullptr, (float *)d_rval, nullptr, nullptr};
+        OrderPlan plan;
+        plan.region[0] = nr <= e->select_order_max ? (int32_t *)region : nullptr;
+        if ((rc = launch_select(e, e->stream, e->counter, e->steal, (const int8_t *)d_rep, nr, 0.f, 0, out, plan))) return rc;
+        TWOPLY_MARK(e, 2);
+        k_twoply_reduce<<<game_grid(e), kGameThreads, kEvalSmem, e->stream>>>(list, e0, e1, rec, (const float *)d_rval, e2, e->fixed);
+        e->launches++;
+        CU(cudaGetLastError());
+        TWOPLY_MARK(e, 3);
+    }
+
+    // 4. the pick
+    k_twoply_pick<<<small_grid, 256, 0, e->stream>>>(queries, n, cnt, off, rec, cmv, clen, expand, e2, nexp, chosen, moves, moves_len, value,
+                                                     n_candidates, n_expanded);
+    e->launches++;
+    CU(cudaGetLastError());
+    TWOPLY_MARK(e, 3);
+    return BGX_OK;
+}
+
+int bgx_select_moves_2ply_host(bgx_engine *e, const int8_t *queries, int64_t n, int32_t max_candidates,
+                               int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value, int32_t *n_candidates, int32_t *n_expanded)
+{
+    USE(e);
+    NEED(queries && n >= 0 && max_candidates >= 0, "bad argument");
+    if (!e->have_weights) { set_error("bgx_select_moves_2ply_host: weights not set"); return BGX_E_STATE; }
+    if (n == 0) return BGX_OK;
+    void *dq, *dc, *dm, *dl, *dv, *dn, *dx;
+    int rc;
+    if ((rc = scratch(e, 0, (size_t)n * 32, &dq))) return rc;
+    if ((rc = scratch(e, 1, (size_t)n * 32, &dc))) return rc;
+    if ((rc = scratch(e, 2, (size_t)n * 8, &dm))) return rc;
+    if ((rc = scratch(e, 3, (size_t)n, &dl))) return rc;
+    if ((rc = scratch(e, 4, (size_t)n * 4, &dv))) return rc;
+    if ((rc = scratch(e, 5, (size_t)n * 4, &dn))) return rc;
+    if ((rc = scratch(e, 6, (size_t)n * 4, &dx))) return rc;
+    CU(cudaMemcpyAsync(dq, queries, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
+    rc = bgx_select_moves_2ply(e, (const int8_t *)dq, n, max_candidates, chosen ? (int8_t *)dc : nullptr, moves ? (int8_t *)dm : nullptr,
+                               moves_len ? (int8_t *)dl : nullptr, value ? (float *)dv : nullptr,
+                               n_candidates ? (int32_t *)dn : nullptr, n_expanded ? (int32_t *)dx : nullptr);
+    if (rc) return rc;
+    if (chosen) CU(cudaMemcpyAsync(chosen, dc, (size_t)n * 32, cudaMemcpyDeviceToHost, e->stream));
+    if (moves) CU(cudaMemcpyAsync(moves, dm, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
+    if (moves_len) CU(cudaMemcpyAsync(moves_len, dl, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+    if (value) CU(cudaMemcpyAsync(value, dv, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+    if (n_candidates) CU(cudaMemcpyAsync(n_candidates, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+    if (n_expanded) CU(cudaMemcpyAsync(n_expanded, dx, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    return BGX_OK;
+}
+
+int bgx_twoply_stage_ms(bgx_engine *e, double *ms)
+{
+    if (!e || !ms) { set_error("bgx_twoply_stage_ms: null"); return BGX_E_INVALID; }
+    for (int k = 0; k < 4; k++) { ms[k] = e->twoply_ms[k]; e->twoply_ms[k] = 0.0; }
     return BGX_OK;
 }
 

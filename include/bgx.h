@@ -173,6 +173,30 @@ int bgx_select_moves_host(bgx_engine *e, const int8_t *queries, int64_t n, float
                           int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value,
                           int32_t *n_seq, int32_t *n_scored);
 
+/* Two-ply move selection: make_move's one-ply rule (model.py:180-222) looking one roll ahead.  Per query (s, mover p, dice):
+ *   candidates   the distinct afterstates of the turn sequences, in order of first appearance in reference order, each with
+ *                the first sequence that reaches it (n_candidates = U of bgx_enumerate_summary);
+ *   a win        a candidate that bears off p's 15th checker is worth exactly 1 (PLAYER1) / 0 (PLAYER2); if there is one, the
+ *                first such candidate is the pick and nothing is expanded;
+ *   filter       max_candidates K = 0 expands every candidate; K > 0 the K best by one-ply value (the value bgx_select_moves
+ *                compares, signed for p; first appearance on ties), so K = 1 picks what bgx_select_moves picks;
+ *   expansion    for each of the opponent's 21 rolls (a = 1..6, b = 1..a, weight 2 if a != b) the reply value R is the value
+ *                bgx_select_moves reports for (A, 1 - p, a, b); a blocked opponent (no sequence, or the empty one of a double)
+ *                leaves V(A, 1 - p), bgx_evaluate's value; E2(A) = sum(weight * R) / 36 in float64, in that roll order, rounded once to fp32;
+ *   pick         arg-max E2 (PLAYER1) / arg-min (PLAYER2), first appearance on ties.
+ * Outputs (any may be NULL) mean what they mean for bgx_select_moves: chosen[n][32] (byte 28 = mover, byte 31 = 1 if a sequence
+ * with a move was played), moves[n][8] / moves_len[n] the first sequence reaching the pick, value[n] its E2 (1 / 0 for a win,
+ * NaN without a sequence), n_candidates[n], n_expanded[n].  A pure function of (query, weights, K).  The replies run through
+ * bgx_select_moves' kernel in chunks of bgx_set_option "twoply_chunk" replies (0 = 2^21), so scratch stays bounded; the device
+ * form synchronises the engine's stream twice to size its buffers.  BGX_E_CAPACITY if a query has more than 4096 distinct
+ * afterstates (never seen: the largest U in 3,200 random games is 783). */
+int bgx_select_moves_2ply(bgx_engine *e, const int8_t *queries, int64_t n, int32_t max_candidates,
+                          int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value,
+                          int32_t *n_candidates, int32_t *n_expanded);
+int bgx_select_moves_2ply_host(bgx_engine *e, const int8_t *queries, int64_t n, int32_t max_candidates,
+                               int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value,
+                               int32_t *n_candidates, int32_t *n_expanded);
+
 /* The same call, asynchronous: copies and kernel are queued on lane `lane`'s own stream
  * (0 <= lane < BGX_ASYNC_LANES) and the call returns at once; bgx_lane_wait(lane) blocks until
  * that lane's outputs are in the host buffers.  Host buffers should be page-locked and must
@@ -343,8 +367,12 @@ int bgx_sfu_monotone(bgx_engine *e, int64_t *ex2_violations, int64_t *rcp_violat
 int bgx_kernel_config(bgx_engine *e, int *selfplay_warps, int *select_warps);
 /* tuning knobs of the fused ply kernels for benchmarks and probes; the defaults are the measured best.  Keys:
  * "selfplay_warps", "select_warps" (16, 20, 24, 32), "select_lane_grid", "select_order_max", "select_urgent_min",
- * "select_giant_min", "select_urgent_from_pct".  The library reads no environment variables. */
+ * "select_giant_min", "select_urgent_from_pct"; for bgx_select_moves_2ply "twoply_chunk" (replies per k_select launch, 0 = 2^21)
+ * and "twoply_timing" (1: time its stages, synchronising between them).  The library reads no environment variables. */
 int bgx_set_option(bgx_engine *e, const char *key, int64_t value);
+/* stage times (ms) accumulated by two-ply calls under "twoply_timing" since the last read: [0] candidates (summary walk, scan,
+ * candidate walk), [1] expansion filter and list, [2] replies (records + k_select), [3] expectation and pick; reset by the read */
+int bgx_twoply_stage_ms(bgx_engine *e, double *ms);
 
 #ifdef __cplusplus
 }
