@@ -244,6 +244,41 @@ class BatchEngine:
                                                 L.ptr(chosen), L.ptr(moves), L.ptr(moves_len), L.ptr(value),
                                                 L.ptr(n_candidates), L.ptr(n_expanded)))
 
+    def rollout_host(self, positions, trials, max_plies=0, seed=0x5EED2026, stratify=True, per_trial=False):
+        """Rollouts (bgx_rollout, DESIGN 7d): `trials` greedy games from every position (int8[n, 32], byte 28 = player on roll),
+        cut after `max_plies` plies (0: played to the end).
+        -> dict(mean f64[n], std_err f64[n], counts int64[n, 8]) and, with per_trial, trial_value f32[n, trials],
+        trial_outcome int8[n, trials], trial_plies int32[n, trials].  counts: outcome classes 1..6 (PLAYER1 single / gammon /
+        backgammon, PLAYER2 the same), truncated trials, plies played."""
+        q = _records(positions)
+        n, trials = q.shape[0], int(trials)
+        o = {"mean": np.zeros(n, np.float64), "std_err": np.zeros(n, np.float64), "counts": np.zeros((n, 8), np.int64)}
+        if per_trial:
+            o["trial_value"] = np.zeros((n, max(trials, 0)), np.float32)
+            o["trial_outcome"] = np.zeros((n, max(trials, 0)), np.int8)
+            o["trial_plies"] = np.zeros((n, max(trials, 0)), np.int32)
+        L.check(self._lib.bgx_rollout_host(self._h, q.ctypes.data, n, trials, int(max_plies), int(seed) & (2 ** 64 - 1),
+                                           L.ROLLOUT_STRATIFY if stratify else 0, L.ptr(o["mean"]), L.ptr(o["std_err"]),
+                                           L.ptr(o["counts"]), L.ptr(o.get("trial_value")), L.ptr(o.get("trial_outcome")),
+                                           L.ptr(o.get("trial_plies"))))
+        return o
+
+    def rollout(self, positions, trials, max_plies=0, seed=0x5EED2026, stratify=True, per_trial=False):
+        """rollout_host on a device tensor of positions: the outputs are device tensors, queued on the engine's stream"""
+        import torch
+        n, trials, dev = positions.shape[0], int(trials), positions.device
+        o = {"mean": torch.empty(n, dtype=torch.float64, device=dev), "std_err": torch.empty(n, dtype=torch.float64, device=dev),
+             "counts": torch.empty((n, 8), dtype=torch.int64, device=dev)}
+        if per_trial:
+            o["trial_value"] = torch.empty((n, max(trials, 0)), dtype=torch.float32, device=dev)
+            o["trial_outcome"] = torch.empty((n, max(trials, 0)), dtype=torch.int8, device=dev)
+            o["trial_plies"] = torch.empty((n, max(trials, 0)), dtype=torch.int32, device=dev)
+        L.check(self._lib.bgx_rollout(self._h, L.ptr(positions), n, trials, int(max_plies), int(seed) & (2 ** 64 - 1),
+                                      L.ROLLOUT_STRATIFY if stratify else 0, L.ptr(o["mean"]), L.ptr(o["std_err"]),
+                                      L.ptr(o["counts"]), L.ptr(o.get("trial_value")), L.ptr(o.get("trial_outcome")),
+                                      L.ptr(o.get("trial_plies"))))
+        return o
+
     def twoply_stage_ms(self):
         """Stage times (ms) of the two-ply calls made since the last read with set_option("twoply_timing", 1):
         candidates, expand, replies, reduce"""

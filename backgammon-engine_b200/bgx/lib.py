@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_PKG, "lib", "libbgx.so")
 
 OK, E_INVALID, E_NO_DEVICE, E_CUDA, E_CAPACITY, E_STATE = 0, -1, -2, -3, -4, -5
 FIRST_ROLLOFF, FIRST_PARITY = 0, 1
+ROLLOUT_STRATIFY, ROLLOUT_MAX_PLIES = 1, 4096
 NPARAMS, NPARAMS_PADDED = 25601, 25604
 
 
@@ -65,7 +66,9 @@ _SIGNATURES = {
     "bgx_select_moves_host": (C.c_int, [_vp, _vp, _i64, C.c_float, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_select_moves_2ply": (C.c_int, [_vp, _vp, _i64, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_select_moves_2ply_host": (C.c_int, [_vp, _vp, _i64, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "bgx_select_moves_host_async": (C.c_int, [_vp, C.c_int, _vp, _i64, C.c_float, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "bgx_rollout": (C.c_int, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_uint64, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "bgx_rollout_host": (C.c_int, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_uint64, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "bgx_select_moves_host_async":(C.c_int, [_vp, C.c_int, _vp, _i64, C.c_float, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_play_ply_host_async": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _i64, C.c_float, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
     "bgx_play_ply_restart_host_async": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _i64, C.c_int, _i64, C.c_float, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
     "bgx_lane_wait": (C.c_int, [_vp, C.c_int]),

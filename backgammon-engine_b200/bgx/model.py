@@ -9,7 +9,8 @@ names and shapes (state_dict compatible with models/*.pth), `learning_rate`, `la
 `make_move`, `initialize_traces`, `initialize_weights`.
 
 Added: `engine()` (a BatchEngine holding these weights), `make_moves_batch` (batched
-make_move over many games at once, greedy or two-ply) — the per-object `make_move` stays a host-side loop because
+make_move over many games at once, greedy or two-ply), `rollout_batch` (rollout values of many
+positions) — the per-object `make_move` stays a host-side loop because
 one position per call cannot amortise a kernel launch; the batch calls are the fast path.
 """
 import random
@@ -182,13 +183,7 @@ class TDLGammonModel(nn.Module):
             raise ValueError(f"plies must be 1 or 2, not {plies}")
         if plies == 2 and epsilon > 0.0:
             raise ValueError("two-ply move selection has no epsilon exploration")
-        q = np.zeros((len(games), 32), np.int8)
-        for i, g in enumerate(games):
-            q[i, :24] = g.getGameBoard()
-            q[i, 24], q[i, 25] = g.getJailedCount(0), g.getJailedCount(1)
-            q[i, 26], q[i, 27] = g.getBornOffCount(0), g.getBornOffCount(1)
-            q[i, 28] = g.getTurn()
-            q[i, 29:31] = g.get_last_dice()
+        q = _game_records(games)
         if plies == 2:
             out = self.engine(device).select_moves_2ply_host(q, max_candidates=candidates)
         else:
@@ -201,3 +196,26 @@ class TDLGammonModel(nn.Module):
                 g.tryMove(mover, abs(o - d), o, d)
             result.append(seq)
         return result
+
+    def rollout_batch(self, games, trials=1296, max_plies=0, seed=0x5EED2026, device=0):
+        """Rollouts of compat Game objects (BatchEngine.rollout_host, DESIGN 7d): `trials` greedy games from each game's
+        position with its player on roll (the dice are ignored), stratified over the first roll when trials is a multiple of 36,
+        cut after `max_plies` plies (0: played to the end).  The games are not modified.
+        -> dict(p1_win f64[n] = P(PLAYER1 wins), std_err f64[n], outcomes f64[n, 6] = fractions of PLAYER1 single / gammon /
+        backgammon and PLAYER2 single / gammon / backgammon wins)"""
+        trials = int(trials)
+        out = self.engine(device).rollout_host(_game_records(games), trials, max_plies=max_plies, seed=seed,
+                                               stratify=trials % 36 == 0)
+        return {"p1_win": out["mean"], "std_err": out["std_err"], "outcomes": out["counts"][:, :6] / float(trials)}
+
+
+def _game_records(games):
+    """RECORDs of compat Game objects: position, player on roll, the dice last rolled"""
+    q = np.zeros((len(games), 32), np.int8)
+    for i, g in enumerate(games):
+        q[i, :24] = g.getGameBoard()
+        q[i, 24], q[i, 25] = g.getJailedCount(0), g.getJailedCount(1)
+        q[i, 26], q[i, 27] = g.getBornOffCount(0), g.getBornOffCount(1)
+        q[i, 28] = g.getTurn()
+        q[i, 29:31] = g.get_last_dice()
+    return q

@@ -289,6 +289,26 @@ class BatchEngine {
         d["chosen"] = chosen; d["moves"] = moves; d["moves_len"] = len; d["value"] = value; d["n_candidates"] = n_cand; d["n_expanded"] = n_exp;
         return d;
     }
+    py::dict rollout(I8 q, int32_t trials, int32_t max_plies, uint64_t seed, bool stratify, bool per_trial)
+    {
+        int64_t n = rows(q);
+        const py::ssize_t T = per_trial && trials > 0 ? trials : 0;
+        py::array_t<double> mean(n), std_err(n);
+        py::array_t<int64_t> counts({(py::ssize_t)n, (py::ssize_t)8});
+        py::array_t<float> value({(py::ssize_t)n, T});
+        py::array_t<int8_t> outcome({(py::ssize_t)n, T});
+        py::array_t<int32_t> plies({(py::ssize_t)n, T});
+        {
+            py::gil_scoped_release nogil;
+            Game::check(bgx_rollout_host(e_, q.data(), n, trials, max_plies, seed, stratify ? BGX_ROLLOUT_STRATIFY : 0, mean.mutable_data(),
+                                         std_err.mutable_data(), counts.mutable_data(), per_trial ? value.mutable_data() : nullptr,
+                                         per_trial ? outcome.mutable_data() : nullptr, per_trial ? plies.mutable_data() : nullptr));
+        }
+        py::dict d;
+        d["mean"] = mean; d["std_err"] = std_err; d["counts"] = counts;
+        if (per_trial) { d["trial_value"] = value; d["trial_outcome"] = outcome; d["trial_plies"] = plies; }
+        return d;
+    }
     py::array_t<float> encode(I8 q)
     {
         int64_t n = rows(q);
@@ -456,6 +476,8 @@ PYBIND11_MODULE(backgammon_env, m)
         .def("evaluate_turn_sequences_summary", &BatchEngine::evaluate_turn_sequences_summary)
         .def("make_moves", &BatchEngine::make_moves, py::arg("queries"), py::arg("epsilon") = 0.0f, py::arg("seed") = 0)
         .def("make_moves_2ply", &BatchEngine::make_moves_2ply, py::arg("queries"), py::arg("max_candidates") = 0)
+        .def("rollout", &BatchEngine::rollout, py::arg("positions"), py::arg("trials"), py::arg("max_plies") = 0,
+             py::arg("seed") = 0x5EED2026ull, py::arg("stratify") = true, py::arg("per_trial") = false)
         .def("encode", &BatchEngine::encode)
         .def("evaluate", &BatchEngine::evaluate)
         .def("get_weights", &BatchEngine::get_weights)

@@ -6,6 +6,7 @@
 #include "bgx_kernels.cuh"
 #include "bgx_td.cuh"
 #include "bgx_twoply.cuh"
+#include "bgx_rollout.cuh"
 
 #include <dlfcn.h>
 
@@ -45,8 +46,8 @@ struct bgx_engine {
     int32_t *fixed = nullptr;     // [198][128] W1 transposed in fixed point (ply kernels, k_evaluate)
     float *aux = nullptr;         // [4] derived scalars: [0] fixed-point scale S, [1] 1/S
     bool have_weights = false;
-    // scratch ([12..] belong to the two-ply path)
-    static constexpr int kScratch = 32;
+    // scratch ([12..31] belong to the two-ply path, [32..] to rollouts)
+    static constexpr int kScratch = 40;
     void *dbuf[kScratch] = {};
     size_t dcap[kScratch] = {};
     unsigned long long *counter = nullptr;   // work queue
@@ -81,6 +82,8 @@ struct bgx_engine {
     long long twoply_chunk = 0;              // replies per k_select launch of a two-ply call (0: kTwoplyChunk)
     bool twoply_timing = false;              // time the stages of a two-ply call (synchronises between them)
     double twoply_ms[4] = {};                // candidates, expand, replies, reduce: accumulated stage times
+    long long rollout_chunk = 0;             // trials (games) per k_rollout launch, whole positions (0: kRolloutChunk)
+    int rollout_warps = 20;                  // warps per CTA of k_rollout
     cudaEvent_t tp0 = nullptr, tp1 = nullptr;
     // bookkeeping
     long long launches = 0;
@@ -180,7 +183,8 @@ static int create_into(bgx_engine *e, int device, const cudaDeviceProp &prop)
     CU(cudaFuncSetAttribute(k_select<W, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));            \
     CU(cudaFuncSetAttribute(k_select<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));             \
     CU(cudaFuncSetAttribute(k_selfplay<W, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));          \
-    CU(cudaFuncSetAttribute(k_selfplay<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));
+    CU(cudaFuncSetAttribute(k_selfplay<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));          \
+    CU(cudaFuncSetAttribute(k_rollout<W, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));
     BGX_SMEM_ATTR(16, 109)
     BGX_SMEM_ATTR(20, 86)
     BGX_SMEM_ATTR(24, 72)
@@ -224,13 +228,15 @@ int bgx_create(int device, bgx_engine **out)
 //   "select_lane_grid"                 CTAs of a launch on an asynchronous lane (0: one per SM; default: half the SMs)
 //   "select_order_max"                 largest batch that gets a sorted queue
 //   "select_urgent_min" / "select_giant_min" / "select_urgent_from_pct"   when a CTA helps a published double
+//   "rollout_warps"                    warps per CTA of k_rollout: 16, 20, 24 or 32
+//   "rollout_chunk"                    trials (games) per k_rollout launch, rounded down to whole positions (0: 2^24)
 int bgx_set_option(bgx_engine *e, const char *key, int64_t value)
 {
     if (!e || !key) { set_error("bgx_set_option: null"); return BGX_E_INVALID; }
     const std::string k(key);
-    if (k == "selfplay_warps" || k == "select_warps") {
+    if (k == "selfplay_warps" || k == "select_warps" || k == "rollout_warps") {
         if (value != 16 && value != 20 && value != 24 && value != 32) { set_error("bgx_set_option: %s must be 16, 20, 24 or 32", key); return BGX_E_INVALID; }
-        (k == "selfplay_warps" ? e->selfplay_warps : e->select_warps) = (int)value;
+        (k == "selfplay_warps" ? e->selfplay_warps : k == "select_warps" ? e->select_warps : e->rollout_warps) = (int)value;
     } else if (k == "select_lane_grid") {
         if (value < 0 || value > e->sm_count) { set_error("bgx_set_option: select_lane_grid is 0 .. %d", e->sm_count); return BGX_E_INVALID; }
         e->lane_grid = (int)value;
@@ -242,6 +248,10 @@ int bgx_set_option(bgx_engine *e, const char *key, int64_t value)
         if (value < 0) { set_error("bgx_set_option: twoply_chunk must be >= 0"); return BGX_E_INVALID; }
         e->twoply_chunk = (long long)value;
     } else if (k == "twoply_timing") e->twoply_timing = value != 0;
+    else if (k == "rollout_chunk") {
+        if (value < 0) { set_error("bgx_set_option: rollout_chunk must be >= 0"); return BGX_E_INVALID; }
+        e->rollout_chunk = (long long)value;
+    }
     else { set_error("bgx_set_option: unknown option '%s'", key); return BGX_E_INVALID; }
     return BGX_OK;
 }
@@ -812,6 +822,100 @@ int bgx_twoply_stage_ms(bgx_engine *e, double *ms)
 {
     if (!e || !ms) { set_error("bgx_twoply_stage_ms: null"); return BGX_E_INVALID; }
     for (int k = 0; k < 4; k++) { ms[k] = e->twoply_ms[k]; e->twoply_ms[k] = 0.0; }
+    return BGX_OK;
+}
+
+// ------------------------------------------------------------------------ rollouts (DESIGN 7d)
+
+constexpr long long kRolloutChunk = 1ll << 24;  // trials per k_rollout launch: 36 MB of per-trial scratch
+
+static int rollout_args(int64_t n, int32_t trials, int32_t max_plies, int flags, const char *who)
+{
+    if (n < 0 || trials < 1) { set_error("%s: n must be >= 0 and trials >= 1", who); return BGX_E_INVALID; }
+    if (max_plies < 0 || max_plies > BGX_ROLLOUT_MAX_PLIES) { set_error("%s: max_plies must be 0 .. %d", who, BGX_ROLLOUT_MAX_PLIES); return BGX_E_INVALID; }
+    if (flags & ~BGX_ROLLOUT_STRATIFY) { set_error("%s: unknown flags 0x%x", who, flags); return BGX_E_INVALID; }
+    if ((flags & BGX_ROLLOUT_STRATIFY) && trials % 36 != 0) { set_error("%s: a stratified rollout needs a multiple of 36 trials", who); return BGX_E_INVALID; }
+    return BGX_OK;
+}
+
+int bgx_rollout(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                double *mean, double *std_err, int64_t *counts, float *trial_value, int8_t *trial_outcome, int32_t *trial_plies)
+{
+    USE(e);
+    if (int rc = rollout_args(n, trials, max_plies, flags, "bgx_rollout")) return rc;
+    NEED(positions || n == 0, "null positions");
+    if (!e->have_weights) { set_error("bgx_rollout: weights not set"); return BGX_E_STATE; }
+    if (n == 0) return BGX_OK;
+    // chunks of whole positions; the per-trial results of a chunk go to the caller's arrays or to engine scratch
+    const long long chunk = e->rollout_chunk > 0 ? e->rollout_chunk : kRolloutChunk;
+    const long long per_launch = std::max<long long>(1, chunk / trials);
+    const long long items_cap = std::min<long long>(n, per_launch) * trials;
+    void *sv = nullptr, *so = nullptr, *sp = nullptr;
+    int rc;
+    if (!trial_value && (rc = scratch(e, 32, (size_t)items_cap * 4, &sv))) return rc;
+    if (!trial_outcome && (rc = scratch(e, 33, (size_t)items_cap, &so))) return rc;
+    if (!trial_plies && (rc = scratch(e, 34, (size_t)items_cap * 4, &sp))) return rc;
+    RolloutParams p;
+    p.trials = trials;
+    p.cap = max_plies > 0 ? max_plies : BGX_ROLLOUT_MAX_PLIES;
+    p.stratify = (flags & BGX_ROLLOUT_STRATIFY) ? 1 : 0;
+    p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
+    p.counter = e->counter; p.zstash = e->zstash;
+    tick(e);
+    for (long long q0 = 0; q0 < n; q0 += per_launch) {
+        const long long np = std::min<long long>(n - q0, per_launch);
+        const size_t at = (size_t)q0 * trials;
+        p.positions = positions + q0 * 32;
+        p.n_items = np * trials;
+        p.value = trial_value ? trial_value + at : (float *)sv;
+        p.outcome = trial_outcome ? trial_outcome + at : (int8_t *)so;
+        p.plies = trial_plies ? trial_plies + at : (int32_t *)sp;
+        CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
+#define BGX_LAUNCH_ROLLOUT(W, S) k_rollout<W, S><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, e->fixed, e->steal)
+        if (e->rollout_warps == 16) BGX_LAUNCH_ROLLOUT(16, 109);
+        else if (e->rollout_warps == 20) BGX_LAUNCH_ROLLOUT(20, 86);
+        else if (e->rollout_warps == 24) BGX_LAUNCH_ROLLOUT(24, 72);
+        else BGX_LAUNCH_ROLLOUT(32, 53);
+#undef BGX_LAUNCH_ROLLOUT
+        if (mean || std_err || counts)
+            k_rollout_reduce<<<(unsigned)((np + 127) / 128), 128, 0, e->stream>>>(p.value, p.outcome, p.plies, np, trials, mean ? mean + q0 : nullptr,
+                                                                              std_err ? std_err + q0 : nullptr,
+                                                                              counts ? (long long *)counts + q0 * 8 : nullptr);
+        e->launches += 2;
+        CU(cudaGetLastError());
+    }
+    tock(e);
+    return BGX_OK;
+}
+
+int bgx_rollout_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                     double *mean, double *std_err, int64_t *counts, float *trial_value, int8_t *trial_outcome, int32_t *trial_plies)
+{
+    USE(e);
+    if (int rc = rollout_args(n, trials, max_plies, flags, "bgx_rollout_host")) return rc;
+    NEED(positions || n == 0, "null positions");
+    if (!e->have_weights) { set_error("bgx_rollout_host: weights not set"); return BGX_E_STATE; }
+    if (n == 0) return BGX_OK;
+    const size_t items = (size_t)n * trials;
+    void *dq, *dm = nullptr, *ds = nullptr, *dc = nullptr, *dv = nullptr, *dout = nullptr, *dp = nullptr;
+    int rc;
+    if ((rc = scratch(e, 35, (size_t)n * 32, &dq))) return rc;
+    if (mean && (rc = scratch(e, 36, (size_t)n * 8, &dm))) return rc;
+    if (std_err && (rc = scratch(e, 37, (size_t)n * 8, &ds))) return rc;
+    if (counts && (rc = scratch(e, 38, (size_t)n * 64, &dc))) return rc;
+    if (trial_value && (rc = scratch(e, 39, items * 4, &dv))) return rc;
+    if (trial_outcome && (rc = scratch(e, 0, items, &dout))) return rc;
+    if (trial_plies && (rc = scratch(e, 1, items * 4, &dp))) return rc;
+    CU(cudaMemcpyAsync(dq, positions, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
+    if ((rc = bgx_rollout(e, (const int8_t *)dq, n, trials, max_plies, seed, flags, (double *)dm, (double *)ds, (int64_t *)dc,
+                          (float *)dv, (int8_t *)dout, (int32_t *)dp))) return rc;
+    if (mean) CU(cudaMemcpyAsync(mean, dm, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
+    if (std_err) CU(cudaMemcpyAsync(std_err, ds, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
+    if (counts) CU(cudaMemcpyAsync(counts, dc, (size_t)n * 64, cudaMemcpyDeviceToHost, e->stream));
+    if (trial_value) CU(cudaMemcpyAsync(trial_value, dv, items * 4, cudaMemcpyDeviceToHost, e->stream));
+    if (trial_outcome) CU(cudaMemcpyAsync(trial_outcome, dout, items, cudaMemcpyDeviceToHost, e->stream));
+    if (trial_plies) CU(cudaMemcpyAsync(trial_plies, dp, items * 4, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
     return BGX_OK;
 }
 

@@ -197,6 +197,39 @@ int bgx_select_moves_2ply_host(bgx_engine *e, const int8_t *queries, int64_t n, 
                                int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value,
                                int32_t *n_candidates, int32_t *n_expanded);
 
+/* Rollouts: Monte Carlo evaluation of n positions (RECORDs: bytes 0..27 the position, byte 28 the player on roll, bytes 29..31
+ * ignored) with bgx_select_moves' greedy one-ply policy (epsilon 0, make_move) on both sides.  Per position, `trials` independent
+ * trials t = 0 .. trials-1, each played until the game ends or `max_plies` plies were played (0: to the end, with the hard cap
+ * BGX_ROLLOUT_MAX_PLIES applied the same way):
+ *   dice       ply k of trial t (k = 0: the player on roll) rolls Philox4x32-10, key = seed, counter = (k, t lo, t hi, 4), dice as
+ *              self-play draws them; with BGX_ROLLOUT_STRATIFY ply 0 rolls r = t mod 36 instead (d1 = 1 + r / 6, d2 = 1 + r % 6), and
+ *              trials must be a multiple of 36.  Dice depend on the trial index only: every position of a batch sees the same dice
+ *              (common random numbers), and results do not depend on batching;
+ *   a ply      is bgx_select_moves at epsilon 0; the game is over when byte 26 == 15 (PLAYER1 wins, checked first) or byte 27 == 15;
+ *   x_t        a P(PLAYER1 wins) estimate: exactly 1 / 0 for a finished game; for a truncated one the value bgx_select_moves reports
+ *              for the last ply played, or V(position, mover) as bgx_evaluate gives it when that ply had no sequence (or only the
+ *              empty sequence of a blocked double);
+ *   outcome    class of a finished trial from its final board: 1 / 2 / 3 PLAYER1 single / gammon (the loser bore nothing off) /
+ *              backgammon (a gammon with a loser's checker on the bar or in the winner's home board), 4 / 5 / 6 the same for
+ *              PLAYER2, 0 truncated.  Reported only: outcomes never change play or the mean.
+ * Outputs, any may be NULL: mean[n] = sum x_t / trials, std_err[n] = sqrt(sum (x_t - mean)^2 / (trials (trials - 1))) (NaN for
+ * one trial; with stratification this plain formula overestimates the error), both float64 and summed sequentially in trial
+ * order; counts[n][8] = trials of outcome class 1..6, truncated trials, plies played in all trials.  The per-trial arrays
+ * trial_value[n][trials], trial_outcome[n][trials], trial_plies[n][trials] are for analysis; without them the per-trial results
+ * live in engine scratch.  A pure function of (position, mover, trials, max_plies, seed, flags, weights): batch composition,
+ * order, chunking (bgx_set_option "rollout_chunk": trials per launch, rounded down to whole positions, 0 = 2^24) and warps per
+ * CTA ("rollout_warps") change nothing.  BGX_E_INVALID for trials < 1, max_plies outside [0, BGX_ROLLOUT_MAX_PLIES], unknown
+ * flags or a stratified rollout whose trials are not a multiple of 36.  The device form queues its work on the engine's stream;
+ * the host form copies in, runs and copies out with one synchronisation. */
+#define BGX_ROLLOUT_STRATIFY 1
+#define BGX_ROLLOUT_MAX_PLIES 4096
+int bgx_rollout(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                double *mean, double *std_err, int64_t *counts,
+                float *trial_value, int8_t *trial_outcome, int32_t *trial_plies);
+int bgx_rollout_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                     double *mean, double *std_err, int64_t *counts,
+                     float *trial_value, int8_t *trial_outcome, int32_t *trial_plies);
+
 /* The same call, asynchronous: copies and kernel are queued on lane `lane`'s own stream
  * (0 <= lane < BGX_ASYNC_LANES) and the call returns at once; bgx_lane_wait(lane) blocks until
  * that lane's outputs are in the host buffers.  Host buffers should be page-locked and must
