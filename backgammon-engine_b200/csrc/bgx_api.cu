@@ -15,9 +15,65 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 using namespace bgx;
+
+#define CU(call)                                                                              \
+    do {                                                                                      \
+        cudaError_t err__ = (call);                                                           \
+        if (err__ != cudaSuccess) {                                                           \
+            set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(err__)); \
+            return BGX_E_CUDA;                                                                \
+        }                                                                                     \
+    } while (0)
+
+#define NEED(cond, msg)                                   \
+    do {                                                  \
+        if (!(cond)) { set_error("%s: %s", __func__, msg); return BGX_E_INVALID; } \
+    } while (0)
+
+// device buffers that are kept from call to call and grow on demand
+template <int K>
+struct Arena {
+    void *buf[K] = {};
+    size_t cap[K] = {};
+
+    // buffer i with room for `bytes`; a buffer too small is freed and reallocated with headroom, its contents lost
+    template <typename T>
+    int grow(int i, size_t bytes, T **out)
+    {
+        if (cap[i] < bytes) {
+            if (buf[i]) CU(cudaFree(buf[i]));
+            buf[i] = nullptr;
+            cap[i] = 0;
+            const size_t want = bytes + bytes / 4 + 256;
+            CU(cudaMalloc(&buf[i], want));
+            cap[i] = want;
+        }
+        *out = static_cast<T *>(buf[i]);
+        return BGX_OK;
+    }
+    void release() { for (void *b : buf) cudaFree(b); }
+};
+
+// the work buffers of the device-form entry points, by name
+enum Work {
+    kSelectOrder,                                    // bgx_select_moves: sorted queue
+    kEnumScanSums,                                   // bgx_enumerate_count: tile sums of the scan
+    // bgx_select_moves_2ply, per query: summary walk, candidate counts and offsets, expansion counts and offsets
+    kTpSeq, kTpUnique, kTpDigest, kTpCount, kTpOffsets, kTpScanSums, kTpFlags, kTpExpandCount, kTpExpandOffsets,
+    // per candidate: record, first sequence, one-ply value, expanded?, two-ply value; the list of expanded candidates
+    kTpRecords, kTpMoves, kTpMovesLen, kTpValue, kTpExpand, kTpE2, kTpList,
+    // per chunk of replies: records, values, sorted queue
+    kTpReplies, kTpReplyValue, kTpReplyOrder,
+    // bgx_rollout: the per-trial results of a chunk the caller did not ask for
+    kRolloutValue, kRolloutOutcome, kRolloutPlies,
+    kWorkBufs
+};
+enum LaneWork { kLaneOrder0, kLaneOrder1, kLaneWorkBufs };   // a lane's sorted queues: the one read, the one written for the next call
+constexpr int kStageBufs = 7;                    // the most host arrays one *_host call stages
 
 // an asynchronous lane of the batched make_move path: its own stream, work-queue counter,
 // sharing buffer and staging buffers, so that two batches can be in flight at once
@@ -26,8 +82,8 @@ struct bgx_lane {
     cudaEvent_t done = nullptr;
     unsigned long long *counter = nullptr;   // [0] work queue, [8..15] the 16 bucket totals of k_select_order
     StealResult *steal = nullptr;
-    void *buf[11] = {};                      // [7] [10]: sorted queues (two slots), [8] [9]: ply and game id of bgx_play_ply_host_async
-    size_t cap[11] = {};
+    Arena<kLaneWorkBufs> work;
+    Arena<kStageBufs> stage;
     int order_slot = 0;                      // slot holding the queue the previous bgx_play_ply_host_async produced for its successor ...
     int64_t order_n = -1;                    // ... valid for a batch of exactly this many queries (-1: none)
     bool busy = false;
@@ -46,10 +102,8 @@ struct bgx_engine {
     int32_t *fixed = nullptr;     // [198][128] W1 transposed in fixed point (ply kernels, k_evaluate)
     float *aux = nullptr;         // [4] derived scalars: [0] fixed-point scale S, [1] 1/S
     bool have_weights = false;
-    // scratch ([12..31] belong to the two-ply path, [32..] to rollouts)
-    static constexpr int kScratch = 40;
-    void *dbuf[kScratch] = {};
-    size_t dcap[kScratch] = {};
+    Arena<kWorkBufs> work;                   // buffers of the device-form calls (enum Work)
+    Arena<kStageBufs> stage;                 // device copies of the host arrays of the *_host calls (Stage)
     unsigned long long *counter = nullptr;   // work queue
     unsigned long long *stats = nullptr;     // 8 counters
     double *dstats = nullptr;                // TD: sum of squared errors
@@ -92,19 +146,68 @@ struct bgx_engine {
     bgx_lane lanes[kLanes];
 };
 
-#define CU(call)                                                                              \
-    do {                                                                                      \
-        cudaError_t err__ = (call);                                                           \
-        if (err__ != cudaSuccess) {                                                           \
-            set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(err__)); \
-            return BGX_E_CUDA;                                                                \
-        }                                                                                     \
-    } while (0)
+// The host side of a *_host call on the engine's stream or on a lane's.  in() and out() hand out staging buffers in call
+// order from an arena that no device-form call touches, so that they can never alias the buffers of the call they wrap.
+// The first failing CUDA call leaves its message in bgx_last_error and its code in rc; later ones are skipped.
+struct Stage {
+    Arena<kStageBufs> &arena;
+    cudaStream_t stream;
+    bgx_lane *lane;                          // null: the engine's stream
+    int rc = BGX_OK, used = 0, n_back = 0;
+    struct Back { void *host; const void *dev; size_t bytes; } back[kStageBufs];
 
-#define NEED(cond, msg)                                   \
-    do {                                                  \
-        if (!(cond)) { set_error("%s: %s", __func__, msg); return BGX_E_INVALID; } \
-    } while (0)
+    explicit Stage(bgx_engine *e) : arena(e->stage), stream(e->stream), lane(nullptr) {}
+    explicit Stage(bgx_lane &l) : arena(l.stage), stream(l.stream), lane(&l) {}
+
+    template <typename T>
+    T *take(size_t bytes)
+    {
+        T *d = nullptr;
+        if (rc == BGX_OK && used == kStageBufs) { set_error("staging: more than %d buffers", kStageBufs); rc = BGX_E_STATE; }
+        if (rc == BGX_OK) rc = arena.grow(used++, bytes, &d);
+        return d;
+    }
+    int h2d(void *dev, const void *host, size_t bytes) { CU(cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, stream)); return BGX_OK; }
+    // a device copy of `host` (null for a null host pointer)
+    template <typename T>
+    T *in(const T *host, size_t bytes)
+    {
+        if (!host) return nullptr;
+        T *d = take<T>(bytes);
+        if (rc == BGX_OK) rc = h2d(d, host, bytes);
+        return d;
+    }
+    // a device buffer whose contents finish() copies to `host` (null for a null host pointer: the call skips that output)
+    template <typename T>
+    T *out(T *host, size_t bytes)
+    {
+        if (!host) return nullptr;
+        T *d = take<T>(bytes);
+        copy_back(host, d, bytes);
+        return d;
+    }
+    void copy_back(void *host, const void *dev, size_t bytes) { back[n_back++] = {host, dev, bytes}; }
+    // after the device call (its return code is passed through): the copies back, then the stream synchronised, or the
+    // lane marked busy until they are done
+    int finish(int call_rc = BGX_OK)
+    {
+        if (call_rc != BGX_OK) return call_rc;
+        for (int i = 0; i < n_back; i++) CU(cudaMemcpyAsync(back[i].host, back[i].dev, back[i].bytes, cudaMemcpyDeviceToHost, stream));
+        n_back = 0;
+        if (!lane) CU(cudaStreamSynchronize(stream));
+        else {
+            CU(cudaEventRecord(lane->done, stream));
+            lane->busy = true;
+        }
+        return BGX_OK;
+    }
+};
+
+static int need_weights(bgx_engine *e, const char *who)
+{
+    if (!e->have_weights) { set_error("%s: weights not set", who); return BGX_E_STATE; }
+    return BGX_OK;
+}
 
 static int use(bgx_engine *e)
 {
@@ -118,26 +221,20 @@ static int use(bgx_engine *e)
         if (rc__ != BGX_OK) return rc__; \
     } while (0)
 
-static int scratch(bgx_engine *e, int i, size_t bytes, void **out)
-{
-    if (e->dcap[i] < bytes) {
-        if (e->dbuf[i]) CU(cudaFree(e->dbuf[i]));
-        e->dbuf[i] = nullptr;
-        e->dcap[i] = 0;
-        size_t want = bytes + bytes / 4 + 256;
-        CU(cudaMalloc(&e->dbuf[i], want));
-        e->dcap[i] = want;
-    }
-    *out = e->dbuf[i];
-    return BGX_OK;
-}
-
 static int tick_(bgx_engine *e) { CU(cudaEventRecord(e->ev0, e->stream)); return BGX_OK; }
 static int tock_(bgx_engine *e) { CU(cudaEventRecord(e->ev1, e->stream)); e->timed = true; return BGX_OK; }
 #define tick(e) do { const int rc__ = tick_(e); if (rc__ != BGX_OK) return rc__; } while (0)
 #define tock(e) do { const int rc__ = tock_(e); if (rc__ != BGX_OK) return rc__; } while (0)
 
 static int game_grid(bgx_engine *e) { return e->sm_count; }   // persistent: one 16-warp CTA per SM
+
+// f(std::true_type) or f(std::false_type): the kExplore instantiation of a fused ply kernel
+template <typename F>
+static void dispatch_explore(bool explore, F &&f)
+{
+    if (explore) f(std::true_type{});
+    else f(std::false_type{});
+}
 
 extern "C" {
 
@@ -177,19 +274,17 @@ static int create_into(bgx_engine *e, int device, const cudaDeviceProp &prop)
     CU(cudaFuncSetAttribute(k_candidates, cudaFuncAttributeMaxDynamicSharedMemorySize, kEvalSmem));
     CU(cudaFuncSetAttribute(k_twoply_reduce, cudaFuncAttributeMaxDynamicSharedMemorySize, kEvalSmem));
     e->lane_grid = e->sm_count / 2;
-    static_assert(ply_smem<16, 109>() <= 232448 && ply_smem<20, 86>() <= 232448 && ply_smem<24, 72>() <= 232448 && ply_smem<32, 53>() <= 232448,
-                  "fused ply kernels: shared memory per CTA");
-#define BGX_SMEM_ATTR(W, S)                                                                                                    \
-    CU(cudaFuncSetAttribute(k_select<W, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));            \
-    CU(cudaFuncSetAttribute(k_select<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));             \
-    CU(cudaFuncSetAttribute(k_selfplay<W, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));          \
-    CU(cudaFuncSetAttribute(k_selfplay<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));          \
-    CU(cudaFuncSetAttribute(k_rollout<W, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, ply_smem<W, S>()));
-    BGX_SMEM_ATTR(16, 109)
-    BGX_SMEM_ATTR(20, 86)
-    BGX_SMEM_ATTR(24, 72)
-    BGX_SMEM_ATTR(32, 53)
-#undef BGX_SMEM_ATTR
+    static_assert(PlyConfigs::fits(232448), "fused ply kernels: shared memory per CTA");
+    const int rc = PlyConfigs::each([](auto c) {
+        constexpr int W = decltype(c)::kWarps, S = decltype(c)::kSets;
+        CU(cudaFuncSetAttribute(k_select<W, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
+        CU(cudaFuncSetAttribute(k_select<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
+        CU(cudaFuncSetAttribute(k_selfplay<W, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
+        CU(cudaFuncSetAttribute(k_selfplay<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
+        CU(cudaFuncSetAttribute(k_rollout<W, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
+        return BGX_OK;
+    });
+    if (rc) return rc;
     CU(cudaFuncSetAttribute(k_td_replay<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTdSmem));
     CU(cudaFuncSetAttribute(k_td_replay<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTdSmem));
     // the smallest carve-out that holds kTdCtasPerSm games (percent of the SM's 228 KB): the rest of the array is their L1
@@ -235,7 +330,7 @@ int bgx_set_option(bgx_engine *e, const char *key, int64_t value)
     if (!e || !key) { set_error("bgx_set_option: null"); return BGX_E_INVALID; }
     const std::string k(key);
     if (k == "selfplay_warps" || k == "select_warps" || k == "rollout_warps") {
-        if (value != 16 && value != 20 && value != 24 && value != 32) { set_error("bgx_set_option: %s must be 16, 20, 24 or 32", key); return BGX_E_INVALID; }
+        if (!PlyConfigs::has(value)) { set_error("bgx_set_option: %s must be 16, 20, 24 or 32", key); return BGX_E_INVALID; }
         (k == "selfplay_warps" ? e->selfplay_warps : k == "select_warps" ? e->select_warps : e->rollout_warps) = (int)value;
     } else if (k == "select_lane_grid") {
         if (value < 0 || value > e->sm_count) { set_error("bgx_set_option: select_lane_grid is 0 .. %d", e->sm_count); return BGX_E_INVALID; }
@@ -261,7 +356,8 @@ int bgx_destroy(bgx_engine *e)
     if (!e) return BGX_OK;
     cudaSetDevice(e->device);
     cudaDeviceSynchronize();
-    for (int i = 0; i < bgx_engine::kScratch; i++) cudaFree(e->dbuf[i]);
+    e->work.release();
+    e->stage.release();
     cudaFree(e->flat); cudaFree(e->wt); cudaFree(e->fixed); cudaFree(e->aux); cudaFree(e->counter); cudaFree(e->stats); cudaFree(e->dstats); cudaFree(e->steal); cudaFree(e->zstash);
     cudaFree(e->uniq_tables); cudaFree(e->uniq_gens); cudaFree(e->slots); cudaFree(e->traj_pre); cudaFree(e->traj_chosen);
     cudaFree(e->ply); cudaFree(e->game_id); cudaFree(e->td_partial); cudaFree(e->td_delta); cudaFree(e->td_prof); cudaFree(e->td_home); cudaFree(e->td_sched);
@@ -274,7 +370,8 @@ int bgx_destroy(bgx_engine *e)
         if (l.stream) cudaStreamDestroy(l.stream);
         if (l.done) cudaEventDestroy(l.done);
         cudaFree(l.counter); cudaFree(l.steal);
-        for (void *b : l.buf) cudaFree(b);
+        l.work.release();
+        l.stage.release();
     }
     delete e;
     return BGX_OK;
@@ -312,16 +409,29 @@ static int rebuild_table(bgx_engine *e)
     return BGX_OK;
 }
 
+// the flat weight layout [W1[128][198] | b1[128] | w2[128] | b2[1]] and the state_dict tensors
+static void pack_weights(float *flat, const float *W1, const float *b1, const float *w2, const float *b2)
+{
+    std::memcpy(flat, W1, kTableFloats * sizeof(float));
+    std::memcpy(flat + kTableFloats, b1, kHidden * sizeof(float));
+    std::memcpy(flat + kTableFloats + kHidden, w2, kHidden * sizeof(float));
+    flat[kTableFloats + 2 * kHidden] = b2[0];
+}
+static void unpack_weights(const float *flat, float *W1, float *b1, float *w2, float *b2)
+{
+    std::memcpy(W1, flat, kTableFloats * sizeof(float));
+    std::memcpy(b1, flat + kTableFloats, kHidden * sizeof(float));
+    std::memcpy(w2, flat + kTableFloats + kHidden, kHidden * sizeof(float));
+    b2[0] = flat[kTableFloats + 2 * kHidden];
+}
+
 int bgx_set_weights(bgx_engine *e, const float *W1, const float *b1, const float *w2, const float *b2)
 {
     USE(e);
     NEED(W1 && b1 && w2 && b2, "null weight pointer");
     if (int rc = lanes_idle(e, "bgx_set_weights")) return rc;
     std::vector<float> flat(BGX_NPARAMS_PADDED, 0.f);
-    std::memcpy(flat.data(), W1, kTableFloats * sizeof(float));
-    std::memcpy(flat.data() + kTableFloats, b1, kHidden * sizeof(float));
-    std::memcpy(flat.data() + kTableFloats + kHidden, w2, kHidden * sizeof(float));
-    flat[kTableFloats + 2 * kHidden] = b2[0];
+    pack_weights(flat.data(), W1, b1, w2, b2);
     CU(cudaMemcpyAsync(e->flat, flat.data(), flat.size() * sizeof(float), cudaMemcpyHostToDevice, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     e->have_weights = true;
@@ -335,10 +445,7 @@ int bgx_get_weights(bgx_engine *e, float *W1, float *b1, float *w2, float *b2)
     std::vector<float> flat(BGX_NPARAMS_PADDED);
     CU(cudaMemcpyAsync(flat.data(), e->flat, flat.size() * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
-    std::memcpy(W1, flat.data(), kTableFloats * sizeof(float));
-    std::memcpy(b1, flat.data() + kTableFloats, kHidden * sizeof(float));
-    std::memcpy(w2, flat.data() + kTableFloats + kHidden, kHidden * sizeof(float));
-    b2[0] = flat[kTableFloats + 2 * kHidden];
+    unpack_weights(flat.data(), W1, b1, w2, b2);
     return BGX_OK;
 }
 
@@ -382,19 +489,13 @@ int bgx_enumerate_summary_host(bgx_engine *e, const int8_t *queries, int64_t n, 
     USE(e);
     NEED(queries && n_seq && n_unique && digest && n >= 0, "bad argument");
     if (n == 0) return BGX_OK;
-    void *dq, *dn, *du, *dd;
-    int rc;
-    if ((rc = scratch(e, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = scratch(e, 1, (size_t)n * 4, &dn))) return rc;
-    if ((rc = scratch(e, 2, (size_t)n * 4, &du))) return rc;
-    if ((rc = scratch(e, 3, (size_t)n * 8, &dd))) return rc;
-    CU(cudaMemcpyAsync(dq, queries, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
-    if ((rc = bgx_enumerate_summary(e, (const int8_t *)dq, n, (int32_t *)dn, (int32_t *)du, (uint64_t *)dd))) return rc;
-    CU(cudaMemcpyAsync(n_seq, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaMemcpyAsync(n_unique, du, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaMemcpyAsync(digest, dd, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    Stage s(e);
+    const int8_t *dq = s.in(queries, (size_t)n * 32);
+    int32_t *dn = s.out(n_seq, (size_t)n * 4);
+    int32_t *du = s.out(n_unique, (size_t)n * 4);
+    uint64_t *dd = s.out(digest, (size_t)n * 8);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_enumerate_summary(e, dq, n, dn, du, dd));
 }
 
 int bgx_enumerate(bgx_engine *e, const int8_t *queries, int64_t n, const int64_t *offsets,
@@ -413,27 +514,34 @@ int bgx_enumerate(bgx_engine *e, const int8_t *queries, int64_t n, const int64_t
     return BGX_OK;
 }
 
+// exclusive prefix sum of cnt[n] into offsets[n + 1]: three launches
+static int scan_counts(bgx_engine *e, const int32_t *cnt, int64_t n, long long *offsets, long long *sums)
+{
+    const int n_tiles = (int)((n + kScanTile - 1) / kScanTile);
+    k_scan_tiles<<<n_tiles, kScanThreads, 0, e->stream>>>(cnt, n, offsets, sums);
+    k_scan_sums<<<1, 1024, 0, e->stream>>>(sums, n_tiles);
+    k_scan_add<<<(unsigned)((n + kScanThreads - 1) / kScanThreads), kScanThreads, 0, e->stream>>>(offsets, n, sums, n_tiles);
+    e->launches += 3;
+    CU(cudaGetLastError());
+    return BGX_OK;
+}
+
 // sizes of every query's sequence list and their exclusive prefix sum, on the device: the allocation pass of the
-// materialised enumeration (a count-only walk, no dedup table, no digest) + a three-launch scan
+// materialised enumeration (a count-only walk, no dedup table, no digest) + the scan
 int bgx_enumerate_count(bgx_engine *e, const int8_t *queries, int64_t n, int32_t *n_seq, int64_t *offsets)
 {
     USE(e);
     NEED(queries && n_seq && offsets && n >= 0, "bad argument");
     if (n == 0) { CU(cudaMemsetAsync(offsets, 0, 8, e->stream)); return BGX_OK; }
     const int n_tiles = (int)((n + kScanTile - 1) / kScanTile);
-    void *sums;
-    int rc;
-    if ((rc = scratch(e, 9, (size_t)(n_tiles + 1) * 8, &sums))) return rc;
+    long long *sums;
+    if (int rc = e->work.grow(kEnumScanSums, (size_t)(n_tiles + 1) * 8, &sums)) return rc;
     CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
     tick(e);
     k_enumerate_count<<<e->sm_count * 2, kGameThreads, 0, e->stream>>>(queries, n, n_seq, e->counter);
     tock(e);
-    k_scan_tiles<<<n_tiles, kScanThreads, 0, e->stream>>>(n_seq, n, (long long *)offsets, (long long *)sums);
-    k_scan_sums<<<1, 1024, 0, e->stream>>>((long long *)sums, n_tiles);
-    k_scan_add<<<(unsigned)((n + kScanThreads - 1) / kScanThreads), kScanThreads, 0, e->stream>>>((long long *)offsets, n, (const long long *)sums, n_tiles);
-    e->launches += 4;
-    CU(cudaGetLastError());
-    return BGX_OK;
+    e->launches++;
+    return scan_counts(e, n_seq, n, (long long *)offsets, sums);
 }
 
 int bgx_enumerate_host(bgx_engine *e, const int8_t *queries, int64_t n, int64_t cap, int64_t *offsets,
@@ -443,33 +551,26 @@ int bgx_enumerate_host(bgx_engine *e, const int8_t *queries, int64_t n, int64_t 
     NEED(queries && total && n >= 0 && cap >= 0, "bad argument");
     *total = 0;
     if (n == 0) { if (offsets) offsets[0] = 0; return BGX_OK; }
-    void *dq, *dn, *doff;
-    int rc;
-    if ((rc = scratch(e, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = scratch(e, 1, (size_t)n * 4, &dn))) return rc;
-    if ((rc = scratch(e, 4, (size_t)(n + 1) * 8, &doff))) return rc;
-    CU(cudaMemcpyAsync(dq, queries, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
-    if ((rc = bgx_enumerate_count(e, (const int8_t *)dq, n, (int32_t *)dn, (int64_t *)doff))) return rc;
+    Stage s(e);
+    const int8_t *dq = s.in(queries, (size_t)n * 32);
+    int32_t *dn = s.take<int32_t>((size_t)n * 4);
+    int64_t *doff = s.take<int64_t>((size_t)(n + 1) * 8);
+    if (s.rc) return s.rc;
     // the one number the host needs before it can size anything: 8 bytes
     int64_t rows_needed = 0;
-    CU(cudaMemcpyAsync(&rows_needed, (const int64_t *)doff + n, 8, cudaMemcpyDeviceToHost, e->stream));
-    if (offsets) CU(cudaMemcpyAsync(offsets, doff, (size_t)(n + 1) * 8, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
+    s.copy_back(&rows_needed, doff + n, 8);
+    if (offsets) s.copy_back(offsets, doff, (size_t)(n + 1) * 8);
+    if (int rc = s.finish(bgx_enumerate_count(e, dq, n, dn, doff))) return rc;
     *total = rows_needed;
     if (rows_needed > cap) { set_error("bgx_enumerate_host: %lld rows needed, cap %lld", (long long)rows_needed, (long long)cap); return BGX_E_CAPACITY; }
     NEED(seq_moves && seq_len && states, "null output buffer");
     const size_t rows = (size_t)rows_needed;
     if (rows == 0) return BGX_OK;
-    void *dm, *dl, *ds;
-    if ((rc = scratch(e, 5, rows * 8, &dm))) return rc;
-    if ((rc = scratch(e, 6, rows, &dl))) return rc;
-    if ((rc = scratch(e, 7, rows * 32, &ds))) return rc;
-    if ((rc = bgx_enumerate(e, (const int8_t *)dq, n, (const int64_t *)doff, (int8_t *)dm, (int8_t *)dl, (int8_t *)ds))) return rc;
-    CU(cudaMemcpyAsync(seq_moves, dm, rows * 8, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaMemcpyAsync(seq_len, dl, rows, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaMemcpyAsync(states, ds, rows * 32, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    int8_t *dm = s.out(seq_moves, rows * 8);
+    int8_t *dl = s.out(seq_len, rows);
+    int8_t *ds = s.out(states, rows * 32);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_enumerate(e, dq, n, doff, dm, dl, ds));
 }
 
 // ------------------------------------------------------------------------ encode / evaluate
@@ -496,22 +597,18 @@ int bgx_encode_host(bgx_engine *e, const int8_t *records, int64_t n, float *X)
     USE(e);
     NEED(records && X && n >= 0, "bad argument");
     if (n == 0) return BGX_OK;
-    void *dq, *dx;
-    int rc;
-    if ((rc = scratch(e, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = scratch(e, 8, (size_t)n * kFeatures * 4, &dx))) return rc;
-    CU(cudaMemcpyAsync(dq, records, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
-    if ((rc = bgx_encode(e, (const int8_t *)dq, n, (float *)dx))) return rc;
-    CU(cudaMemcpyAsync(X, dx, (size_t)n * kFeatures * 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    Stage s(e);
+    const int8_t *dq = s.in(records, (size_t)n * 32);
+    float *dx = s.out(X, (size_t)n * kFeatures * 4);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_encode(e, dq, n, dx));
 }
 
 int bgx_evaluate(bgx_engine *e, const int8_t *records, int64_t n, float *V)
 {
     USE(e);
     NEED(records && V && n >= 0, "bad argument");
-    if (!e->have_weights) { set_error("bgx_evaluate: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "bgx_evaluate")) return rc;
     if (n == 0) return BGX_OK;
     tick(e);
     k_evaluate<<<game_grid(e), kGameThreads, kEvalSmem, e->stream>>>(records, n, V, e->fixed, e->flat);
@@ -526,15 +623,11 @@ int bgx_evaluate_host(bgx_engine *e, const int8_t *records, int64_t n, float *V)
     USE(e);
     NEED(records && V && n >= 0, "bad argument");
     if (n == 0) return BGX_OK;
-    void *dq, *dv;
-    int rc;
-    if ((rc = scratch(e, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = scratch(e, 1, (size_t)n * 4, &dv))) return rc;
-    CU(cudaMemcpyAsync(dq, records, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
-    if ((rc = bgx_evaluate(e, (const int8_t *)dq, n, (float *)dv))) return rc;
-    CU(cudaMemcpyAsync(V, dv, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    Stage s(e);
+    const int8_t *dq = s.in(records, (size_t)n * 32);
+    float *dv = s.out(V, (size_t)n * 4);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_evaluate(e, dq, n, dv));
 }
 
 // ------------------------------------------------------------------------ batched make_move
@@ -570,15 +663,13 @@ static int launch_select(bgx_engine *e, cudaStream_t stream, unsigned long long 
         CU(cudaMemsetAsync(adv.next_totals, 0, kOrderBuckets * sizeof(uint32_t), stream));
     }
     const SelectTune tune = {(unsigned long long)(n * (int64_t)e->select_urgent_from_pct / 100), e->select_urgent_min, e->select_giant_min};
-#define BGX_LAUNCH_SELECT(W, S, X)                                                                          \
-    k_select<W, S, X><<<grid, W * 32, ply_smem<W, S>(), stream>>>(queries, n, epsilon, (uint32_t)seed, \
-                                                                          (uint32_t)(seed >> 32), out, e->fixed, e->flat, counter, steal, tune, region, totals, adv)
-    const bool ex = epsilon > 0.f;
-    if (e->select_warps == 16) { if (ex) BGX_LAUNCH_SELECT(16, 109, true); else BGX_LAUNCH_SELECT(16, 109, false); }
-    else if (e->select_warps == 20) { if (ex) BGX_LAUNCH_SELECT(20, 86, true); else BGX_LAUNCH_SELECT(20, 86, false); }
-    else if (e->select_warps == 24) { if (ex) BGX_LAUNCH_SELECT(24, 72, true); else BGX_LAUNCH_SELECT(24, 72, false); }
-    else { if (ex) BGX_LAUNCH_SELECT(32, 53, true); else BGX_LAUNCH_SELECT(32, 53, false); }
-#undef BGX_LAUNCH_SELECT
+    PlyConfigs::dispatch(e->select_warps, [&](auto c) {
+        constexpr int W = decltype(c)::kWarps, S = decltype(c)::kSets;
+        dispatch_explore(epsilon > 0.f, [&](auto x) {
+            k_select<W, S, decltype(x)::value><<<grid, W * 32, ply_smem<W, S>(), stream>>>(
+                queries, n, epsilon, (uint32_t)seed, (uint32_t)(seed >> 32), out, e->fixed, e->flat, counter, steal, tune, region, totals, adv);
+        });
+    });
     e->launches++;
     CU(cudaGetLastError());
     return BGX_OK;
@@ -589,16 +680,13 @@ int bgx_select_moves(bgx_engine *e, const int8_t *queries, int64_t n, float epsi
 {
     USE(e);
     NEED(queries && n >= 0, "bad argument");
-    if (!e->have_weights) { set_error("bgx_select_moves: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "bgx_select_moves")) return rc;
     if (n == 0) return BGX_OK;
     const SelectOut out = {chosen, moves, moves_len, value, n_seq, n_scored};
-    void *region = nullptr;
-    if (n <= e->select_order_max) {
-        const int rs = scratch(e, 11, (size_t)n * kOrderBuckets * 4, &region);
-        if (rs) return rs;
-    }
     OrderPlan plan;
-    plan.region[0] = (int32_t *)region;
+    if (n <= e->select_order_max) {
+        if (int rc = e->work.grow(kSelectOrder, (size_t)n * kOrderBuckets * 4, &plan.region[0])) return rc;
+    }
     tick(e);
     const int rc = launch_select(e, e->stream, e->counter, e->steal, queries, n, epsilon, seed, out, plan);
     tock(e);
@@ -611,28 +699,16 @@ int bgx_select_moves_host(bgx_engine *e, const int8_t *queries, int64_t n, float
     USE(e);
     NEED(queries && n >= 0, "bad argument");
     if (n == 0) return BGX_OK;
-    void *dq, *dc, *dm, *dl, *dv, *dn, *ds;
-    int rc;
-    if ((rc = scratch(e, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = scratch(e, 1, (size_t)n * 32, &dc))) return rc;
-    if ((rc = scratch(e, 2, (size_t)n * 8, &dm))) return rc;
-    if ((rc = scratch(e, 3, (size_t)n, &dl))) return rc;
-    if ((rc = scratch(e, 4, (size_t)n * 4, &dv))) return rc;
-    if ((rc = scratch(e, 5, (size_t)n * 4, &dn))) return rc;
-    if ((rc = scratch(e, 6, (size_t)n * 4, &ds))) return rc;
-    CU(cudaMemcpyAsync(dq, queries, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
-    rc = bgx_select_moves(e, (const int8_t *)dq, n, epsilon, seed, chosen ? (int8_t *)dc : nullptr, moves ? (int8_t *)dm : nullptr,
-                          moves_len ? (int8_t *)dl : nullptr, value ? (float *)dv : nullptr,
-                          n_seq ? (int32_t *)dn : nullptr, n_scored ? (int32_t *)ds : nullptr);
-    if (rc) return rc;
-    if (chosen) CU(cudaMemcpyAsync(chosen, dc, (size_t)n * 32, cudaMemcpyDeviceToHost, e->stream));
-    if (moves) CU(cudaMemcpyAsync(moves, dm, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
-    if (moves_len) CU(cudaMemcpyAsync(moves_len, dl, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-    if (value) CU(cudaMemcpyAsync(value, dv, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    if (n_seq) CU(cudaMemcpyAsync(n_seq, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    if (n_scored) CU(cudaMemcpyAsync(n_scored, ds, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    Stage s(e);
+    const int8_t *dq = s.in(queries, (size_t)n * 32);
+    int8_t *dc = s.out(chosen, (size_t)n * 32);
+    int8_t *dm = s.out(moves, (size_t)n * 8);
+    int8_t *dl = s.out(moves_len, (size_t)n);
+    float *dv = s.out(value, (size_t)n * 4);
+    int32_t *dn = s.out(n_seq, (size_t)n * 4);
+    int32_t *ds = s.out(n_scored, (size_t)n * 4);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_select_moves(e, dq, n, epsilon, seed, dc, dm, dl, dv, dn, ds));
 }
 
 // ------------------------------------------------------------------------ two-ply move selection (DESIGN 7c)
@@ -653,24 +729,12 @@ static int twoply_mark(bgx_engine *e, int k)
 }
 #define TWOPLY_MARK(e, k) do { const int rc__ = twoply_mark(e, k); if (rc__ != BGX_OK) return rc__; } while (0)
 
-// exclusive prefix sum of cnt[n] into offsets[n + 1] (the k_scan_* launches of bgx_enumerate_count)
-static int scan_counts(bgx_engine *e, const int32_t *cnt, int64_t n, long long *offsets, long long *sums)
-{
-    const int n_tiles = (int)((n + kScanTile - 1) / kScanTile);
-    k_scan_tiles<<<n_tiles, kScanThreads, 0, e->stream>>>(cnt, n, offsets, sums);
-    k_scan_sums<<<1, 1024, 0, e->stream>>>(sums, n_tiles);
-    k_scan_add<<<(unsigned)((n + kScanThreads - 1) / kScanThreads), kScanThreads, 0, e->stream>>>(offsets, n, sums, n_tiles);
-    e->launches += 3;
-    CU(cudaGetLastError());
-    return BGX_OK;
-}
-
 int bgx_select_moves_2ply(bgx_engine *e, const int8_t *queries, int64_t n, int32_t max_candidates,
                           int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value, int32_t *n_candidates, int32_t *n_expanded)
 {
     USE(e);
     NEED(queries && n >= 0 && max_candidates >= 0, "bad argument");
-    if (!e->have_weights) { set_error("bgx_select_moves_2ply: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "bgx_select_moves_2ply")) return rc;
     if (n == 0) return BGX_OK;
     int rc = ensure_uniq_tables(e);
     if (rc) return rc;
@@ -679,26 +743,25 @@ int bgx_select_moves_2ply(bgx_engine *e, const int8_t *queries, int64_t n, int32
         CU(cudaEventRecord(e->tp0, e->stream));
     }
     const int n_tiles = (int)((n + kScanTile - 1) / kScanTile);
-    void *d_nseq, *d_u, *d_dig, *d_cnt, *d_off, *d_sums, *d_flags, *d_nexp, *d_eoff;
-    if ((rc = scratch(e, 12, (size_t)n * 4, &d_nseq))) return rc;
-    if ((rc = scratch(e, 13, (size_t)n * 4, &d_u))) return rc;
-    if ((rc = scratch(e, 14, (size_t)n * 8, &d_dig))) return rc;
-    if ((rc = scratch(e, 15, (size_t)n * 4, &d_cnt))) return rc;
-    if ((rc = scratch(e, 16, (size_t)(n + 1) * 8, &d_off))) return rc;
-    if ((rc = scratch(e, 17, (size_t)(n_tiles + 1) * 8, &d_sums))) return rc;
-    if ((rc = scratch(e, 18, 16, &d_flags))) return rc;
-    if ((rc = scratch(e, 19, (size_t)n * 4, &d_nexp))) return rc;
-    if ((rc = scratch(e, 20, (size_t)(n + 1) * 8, &d_eoff))) return rc;
-    int32_t *cnt = (int32_t *)d_cnt, *nexp = (int32_t *)d_nexp;
-    long long *off = (long long *)d_off, *eoff = (long long *)d_eoff, *sums = (long long *)d_sums;
-    int *flags = (int *)d_flags;
+    int32_t *nseq, *uniq, *cnt, *nexp;
+    unsigned long long *dig;
+    long long *off, *eoff, *sums;
+    int *flags;
+    if ((rc = e->work.grow(kTpSeq, (size_t)n * 4, &nseq))) return rc;
+    if ((rc = e->work.grow(kTpUnique, (size_t)n * 4, &uniq))) return rc;
+    if ((rc = e->work.grow(kTpDigest, (size_t)n * 8, &dig))) return rc;
+    if ((rc = e->work.grow(kTpCount, (size_t)n * 4, &cnt))) return rc;
+    if ((rc = e->work.grow(kTpOffsets, (size_t)(n + 1) * 8, &off))) return rc;
+    if ((rc = e->work.grow(kTpScanSums, (size_t)(n_tiles + 1) * 8, &sums))) return rc;
+    if ((rc = e->work.grow(kTpFlags, 16, &flags))) return rc;
+    if ((rc = e->work.grow(kTpExpandCount, (size_t)n * 4, &nexp))) return rc;
+    if ((rc = e->work.grow(kTpExpandOffsets, (size_t)(n + 1) * 8, &eoff))) return rc;
 
     // 1. candidates: U per query (the summary walk), their offsets, then every distinct afterstate with its first sequence and V
     CU(cudaMemsetAsync(flags, 0, 16, e->stream));
     CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
-    k_enumerate_summary<<<e->uniq_grid, kGameThreads, 0, e->stream>>>(queries, n, (int32_t *)d_nseq, (int32_t *)d_u,
-                                                                       (unsigned long long *)d_dig, e->uniq_tables, e->uniq_gens, e->counter);
-    k_twoply_count<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>((const int32_t *)d_u, n, cnt, flags);
+    k_enumerate_summary<<<e->uniq_grid, kGameThreads, 0, e->stream>>>(queries, n, nseq, uniq, dig, e->uniq_tables, e->uniq_gens, e->counter);
+    k_twoply_count<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(uniq, n, cnt, flags);
     e->launches += 2;
     if ((rc = scan_counts(e, cnt, n, off, sums))) return rc;
     long long n_cand = 0;
@@ -710,16 +773,15 @@ int bgx_select_moves_2ply(bgx_engine *e, const int8_t *queries, int64_t n, int32
         set_error("bgx_select_moves_2ply: a query has more distinct afterstates than the exact-dedup table holds (%d)", kUniqSlots);
         return BGX_E_CAPACITY;
     }
-    void *d_rec = nullptr, *d_mv = nullptr, *d_len = nullptr, *d_val = nullptr, *d_exp = nullptr, *d_e2 = nullptr;
+    int8_t *rec, *cmv, *clen, *expand;
+    float *val, *e2;
     const size_t C = (size_t)(n_cand > 0 ? n_cand : 1);
-    if ((rc = scratch(e, 21, C * 32, &d_rec))) return rc;
-    if ((rc = scratch(e, 22, C * 8, &d_mv))) return rc;
-    if ((rc = scratch(e, 23, C, &d_len))) return rc;
-    if ((rc = scratch(e, 24, C * 4, &d_val))) return rc;
-    if ((rc = scratch(e, 25, C, &d_exp))) return rc;
-    if ((rc = scratch(e, 26, C * 4, &d_e2))) return rc;
-    int8_t *rec = (int8_t *)d_rec, *cmv = (int8_t *)d_mv, *clen = (int8_t *)d_len, *expand = (int8_t *)d_exp;
-    float *val = (float *)d_val, *e2 = (float *)d_e2;
+    if ((rc = e->work.grow(kTpRecords, C * 32, &rec))) return rc;
+    if ((rc = e->work.grow(kTpMoves, C * 8, &cmv))) return rc;
+    if ((rc = e->work.grow(kTpMovesLen, C, &clen))) return rc;
+    if ((rc = e->work.grow(kTpValue, C * 4, &val))) return rc;
+    if ((rc = e->work.grow(kTpExpand, C, &expand))) return rc;
+    if ((rc = e->work.grow(kTpE2, C * 4, &e2))) return rc;
     if (n_cand > 0) {
         CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
         k_candidates<<<game_grid(e), kGameThreads, kEvalSmem, e->stream>>>(queries, n, cnt, off, rec, cmv, clen, val, e->uniq_tables,
@@ -742,9 +804,8 @@ int bgx_select_moves_2ply(bgx_engine *e, const int8_t *queries, int64_t n, int32
         set_error("bgx_select_moves_2ply: the candidate walk disagreed with the summary walk");
         return BGX_E_CUDA;
     }
-    void *d_list = nullptr;
-    if ((rc = scratch(e, 27, (size_t)(n_exp > 0 ? n_exp : 1) * 8, &d_list))) return rc;
-    long long *list = (long long *)d_list;
+    long long *list;
+    if ((rc = e->work.grow(kTpList, (size_t)(n_exp > 0 ? n_exp : 1) * 8, &list))) return rc;
     if (n_exp > 0) {
         k_twoply_list<<<small_grid, 256, 0, e->stream>>>(n, cnt, off, expand, eoff, list);
         e->launches++;
@@ -755,24 +816,25 @@ int bgx_select_moves_2ply(bgx_engine *e, const int8_t *queries, int64_t n, int32
     const long long chunk_replies = std::max<long long>(e->twoply_chunk > 0 ? e->twoply_chunk : kTwoplyChunk, kRolls);
     const long long per_chunk = chunk_replies / kRolls;
     const long long cap_replies = std::min<long long>(n_exp, per_chunk) * kRolls;
-    void *d_rep = nullptr, *d_rval = nullptr, *region = nullptr;
+    int8_t *rep = nullptr;
+    float *rval = nullptr;
+    int32_t *region = nullptr;
     if (n_exp > 0) {
-        if ((rc = scratch(e, 28, (size_t)cap_replies * 32, &d_rep))) return rc;
-        if ((rc = scratch(e, 29, (size_t)cap_replies * 4, &d_rval))) return rc;
-        if (cap_replies <= e->select_order_max && (rc = scratch(e, 30, (size_t)cap_replies * kOrderBuckets * 4, &region))) return rc;
+        if ((rc = e->work.grow(kTpReplies, (size_t)cap_replies * 32, &rep))) return rc;
+        if ((rc = e->work.grow(kTpReplyValue, (size_t)cap_replies * 4, &rval))) return rc;
+        if (cap_replies <= e->select_order_max && (rc = e->work.grow(kTpReplyOrder, (size_t)cap_replies * kOrderBuckets * 4, &region))) return rc;
     }
     for (long long e0 = 0; e0 < n_exp; e0 += per_chunk) {
         const long long e1 = std::min(n_exp, e0 + per_chunk);
         const long long nr = (e1 - e0) * kRolls;
-        k_twoply_replies<<<(unsigned)std::min<long long>((nr + 7) / 8, (long long)e->sm_count * 16), 256, 0, e->stream>>>(list, e0, nr, rec,
-                                                                                                                        (int8_t *)d_rep);
+        k_twoply_replies<<<(unsigned)std::min<long long>((nr + 7) / 8, (long long)e->sm_count * 16), 256, 0, e->stream>>>(list, e0, nr, rec, rep);
         e->launches++;
-        const SelectOut out = {nullptr, nullptr, nullptr, (float *)d_rval, nullptr, nullptr};
+        const SelectOut out = {nullptr, nullptr, nullptr, rval, nullptr, nullptr};
         OrderPlan plan;
-        plan.region[0] = nr <= e->select_order_max ? (int32_t *)region : nullptr;
-        if ((rc = launch_select(e, e->stream, e->counter, e->steal, (const int8_t *)d_rep, nr, 0.f, 0, out, plan))) return rc;
+        plan.region[0] = nr <= e->select_order_max ? region : nullptr;
+        if ((rc = launch_select(e, e->stream, e->counter, e->steal, rep, nr, 0.f, 0, out, plan))) return rc;
         TWOPLY_MARK(e, 2);
-        k_twoply_reduce<<<game_grid(e), kGameThreads, kEvalSmem, e->stream>>>(list, e0, e1, rec, (const float *)d_rval, e2, e->fixed);
+        k_twoply_reduce<<<game_grid(e), kGameThreads, kEvalSmem, e->stream>>>(list, e0, e1, rec, rval, e2, e->fixed);
         e->launches++;
         CU(cudaGetLastError());
         TWOPLY_MARK(e, 3);
@@ -792,30 +854,18 @@ int bgx_select_moves_2ply_host(bgx_engine *e, const int8_t *queries, int64_t n, 
 {
     USE(e);
     NEED(queries && n >= 0 && max_candidates >= 0, "bad argument");
-    if (!e->have_weights) { set_error("bgx_select_moves_2ply_host: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "bgx_select_moves_2ply_host")) return rc;
     if (n == 0) return BGX_OK;
-    void *dq, *dc, *dm, *dl, *dv, *dn, *dx;
-    int rc;
-    if ((rc = scratch(e, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = scratch(e, 1, (size_t)n * 32, &dc))) return rc;
-    if ((rc = scratch(e, 2, (size_t)n * 8, &dm))) return rc;
-    if ((rc = scratch(e, 3, (size_t)n, &dl))) return rc;
-    if ((rc = scratch(e, 4, (size_t)n * 4, &dv))) return rc;
-    if ((rc = scratch(e, 5, (size_t)n * 4, &dn))) return rc;
-    if ((rc = scratch(e, 6, (size_t)n * 4, &dx))) return rc;
-    CU(cudaMemcpyAsync(dq, queries, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
-    rc = bgx_select_moves_2ply(e, (const int8_t *)dq, n, max_candidates, chosen ? (int8_t *)dc : nullptr, moves ? (int8_t *)dm : nullptr,
-                               moves_len ? (int8_t *)dl : nullptr, value ? (float *)dv : nullptr,
-                               n_candidates ? (int32_t *)dn : nullptr, n_expanded ? (int32_t *)dx : nullptr);
-    if (rc) return rc;
-    if (chosen) CU(cudaMemcpyAsync(chosen, dc, (size_t)n * 32, cudaMemcpyDeviceToHost, e->stream));
-    if (moves) CU(cudaMemcpyAsync(moves, dm, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
-    if (moves_len) CU(cudaMemcpyAsync(moves_len, dl, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-    if (value) CU(cudaMemcpyAsync(value, dv, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    if (n_candidates) CU(cudaMemcpyAsync(n_candidates, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    if (n_expanded) CU(cudaMemcpyAsync(n_expanded, dx, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    Stage s(e);
+    const int8_t *dq = s.in(queries, (size_t)n * 32);
+    int8_t *dc = s.out(chosen, (size_t)n * 32);
+    int8_t *dm = s.out(moves, (size_t)n * 8);
+    int8_t *dl = s.out(moves_len, (size_t)n);
+    float *dv = s.out(value, (size_t)n * 4);
+    int32_t *dn = s.out(n_candidates, (size_t)n * 4);
+    int32_t *dx = s.out(n_expanded, (size_t)n * 4);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_select_moves_2ply(e, dq, n, max_candidates, dc, dm, dl, dv, dn, dx));
 }
 
 int bgx_twoply_stage_ms(bgx_engine *e, double *ms)
@@ -844,17 +894,19 @@ int bgx_rollout(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trial
     USE(e);
     if (int rc = rollout_args(n, trials, max_plies, flags, "bgx_rollout")) return rc;
     NEED(positions || n == 0, "null positions");
-    if (!e->have_weights) { set_error("bgx_rollout: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "bgx_rollout")) return rc;
     if (n == 0) return BGX_OK;
-    // chunks of whole positions; the per-trial results of a chunk go to the caller's arrays or to engine scratch
+    // chunks of whole positions; the per-trial results of a chunk go to the caller's arrays or to engine work buffers
     const long long chunk = e->rollout_chunk > 0 ? e->rollout_chunk : kRolloutChunk;
     const long long per_launch = std::max<long long>(1, chunk / trials);
     const long long items_cap = std::min<long long>(n, per_launch) * trials;
-    void *sv = nullptr, *so = nullptr, *sp = nullptr;
+    float *sv = nullptr;
+    int8_t *so = nullptr;
+    int32_t *sp = nullptr;
     int rc;
-    if (!trial_value && (rc = scratch(e, 32, (size_t)items_cap * 4, &sv))) return rc;
-    if (!trial_outcome && (rc = scratch(e, 33, (size_t)items_cap, &so))) return rc;
-    if (!trial_plies && (rc = scratch(e, 34, (size_t)items_cap * 4, &sp))) return rc;
+    if (!trial_value && (rc = e->work.grow(kRolloutValue, (size_t)items_cap * 4, &sv))) return rc;
+    if (!trial_outcome && (rc = e->work.grow(kRolloutOutcome, (size_t)items_cap, &so))) return rc;
+    if (!trial_plies && (rc = e->work.grow(kRolloutPlies, (size_t)items_cap * 4, &sp))) return rc;
     RolloutParams p;
     p.trials = trials;
     p.cap = max_plies > 0 ? max_plies : BGX_ROLLOUT_MAX_PLIES;
@@ -867,16 +919,14 @@ int bgx_rollout(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trial
         const size_t at = (size_t)q0 * trials;
         p.positions = positions + q0 * 32;
         p.n_items = np * trials;
-        p.value = trial_value ? trial_value + at : (float *)sv;
-        p.outcome = trial_outcome ? trial_outcome + at : (int8_t *)so;
-        p.plies = trial_plies ? trial_plies + at : (int32_t *)sp;
+        p.value = trial_value ? trial_value + at : sv;
+        p.outcome = trial_outcome ? trial_outcome + at : so;
+        p.plies = trial_plies ? trial_plies + at : sp;
         CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
-#define BGX_LAUNCH_ROLLOUT(W, S) k_rollout<W, S><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, e->fixed, e->steal)
-        if (e->rollout_warps == 16) BGX_LAUNCH_ROLLOUT(16, 109);
-        else if (e->rollout_warps == 20) BGX_LAUNCH_ROLLOUT(20, 86);
-        else if (e->rollout_warps == 24) BGX_LAUNCH_ROLLOUT(24, 72);
-        else BGX_LAUNCH_ROLLOUT(32, 53);
-#undef BGX_LAUNCH_ROLLOUT
+        PlyConfigs::dispatch(e->rollout_warps, [&](auto c) {
+            constexpr int W = decltype(c)::kWarps, S = decltype(c)::kSets;
+            k_rollout<W, S><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, e->fixed, e->steal);
+        });
         if (mean || std_err || counts)
             k_rollout_reduce<<<(unsigned)((np + 127) / 128), 128, 0, e->stream>>>(p.value, p.outcome, p.plies, np, trials, mean ? mean + q0 : nullptr,
                                                                               std_err ? std_err + q0 : nullptr,
@@ -894,103 +944,27 @@ int bgx_rollout_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t 
     USE(e);
     if (int rc = rollout_args(n, trials, max_plies, flags, "bgx_rollout_host")) return rc;
     NEED(positions || n == 0, "null positions");
-    if (!e->have_weights) { set_error("bgx_rollout_host: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "bgx_rollout_host")) return rc;
     if (n == 0) return BGX_OK;
     const size_t items = (size_t)n * trials;
-    void *dq, *dm = nullptr, *ds = nullptr, *dc = nullptr, *dv = nullptr, *dout = nullptr, *dp = nullptr;
-    int rc;
-    if ((rc = scratch(e, 35, (size_t)n * 32, &dq))) return rc;
-    if (mean && (rc = scratch(e, 36, (size_t)n * 8, &dm))) return rc;
-    if (std_err && (rc = scratch(e, 37, (size_t)n * 8, &ds))) return rc;
-    if (counts && (rc = scratch(e, 38, (size_t)n * 64, &dc))) return rc;
-    if (trial_value && (rc = scratch(e, 39, items * 4, &dv))) return rc;
-    if (trial_outcome && (rc = scratch(e, 0, items, &dout))) return rc;
-    if (trial_plies && (rc = scratch(e, 1, items * 4, &dp))) return rc;
-    CU(cudaMemcpyAsync(dq, positions, (size_t)n * 32, cudaMemcpyHostToDevice, e->stream));
-    if ((rc = bgx_rollout(e, (const int8_t *)dq, n, trials, max_plies, seed, flags, (double *)dm, (double *)ds, (int64_t *)dc,
-                          (float *)dv, (int8_t *)dout, (int32_t *)dp))) return rc;
-    if (mean) CU(cudaMemcpyAsync(mean, dm, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
-    if (std_err) CU(cudaMemcpyAsync(std_err, ds, (size_t)n * 8, cudaMemcpyDeviceToHost, e->stream));
-    if (counts) CU(cudaMemcpyAsync(counts, dc, (size_t)n * 64, cudaMemcpyDeviceToHost, e->stream));
-    if (trial_value) CU(cudaMemcpyAsync(trial_value, dv, items * 4, cudaMemcpyDeviceToHost, e->stream));
-    if (trial_outcome) CU(cudaMemcpyAsync(trial_outcome, dout, items, cudaMemcpyDeviceToHost, e->stream));
-    if (trial_plies) CU(cudaMemcpyAsync(trial_plies, dp, items * 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    Stage s(e);
+    const int8_t *dq = s.in(positions, (size_t)n * 32);
+    double *dm = s.out(mean, (size_t)n * 8);
+    double *ds = s.out(std_err, (size_t)n * 8);
+    int64_t *dc = s.out(counts, (size_t)n * 64);
+    float *dv = s.out(trial_value, items * 4);
+    int8_t *dout = s.out(trial_outcome, items);
+    int32_t *dp = s.out(trial_plies, items * 4);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_rollout(e, dq, n, trials, max_plies, seed, flags, dm, ds, dc, dv, dout, dp));
 }
 
-// Asynchronous form of bgx_select_moves_host: the copies and the kernel are queued on lane `lane`'s own
-// stream and the call returns; bgx_lane_wait blocks until that lane's results are in the host buffers.
-// A few lanes in flight let the host advance one part of a population while the GPU plays the others.
-static int lane_scratch(bgx_lane &l, int i, size_t bytes, void **out)
+// the start of a call on lane `lane`: the lane is free, its stream and buffers exist, and its stream waits for the work
+// queued on the engine's stream so far (weights set before the call are visible to the lane)
+static int lane_begin(bgx_engine *e, int lane, const char *who, bgx_lane **out)
 {
-    if (l.cap[i] < bytes) {
-        if (l.buf[i]) CU(cudaFree(l.buf[i]));
-        l.buf[i] = nullptr;
-        l.cap[i] = 0;
-        const size_t want = bytes + bytes / 4 + 256;
-        CU(cudaMalloc(&l.buf[i], want));
-        l.cap[i] = want;
-    }
-    *out = l.buf[i];
-    return BGX_OK;
-}
-
-int bgx_select_moves_host_async(bgx_engine *e, int lane, const int8_t *queries, int64_t n, float epsilon, uint64_t seed,
-                                int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value, int32_t *n_seq, int32_t *n_scored)
-{
-    USE(e);
-    NEED(lane >= 0 && lane < kLanes, "lane out of range");
-    NEED(queries && n >= 0, "bad argument");
-    if (!e->have_weights) { set_error("bgx_select_moves_host_async: weights not set"); return BGX_E_STATE; }
-    bgx_lane &l = e->lanes[lane];
-    if (l.busy) { set_error("bgx_select_moves_host_async: lane %d has a batch in flight (bgx_lane_wait first)", lane); return BGX_E_STATE; }
-    if (!l.stream) {
-        CU(cudaStreamCreateWithFlags(&l.stream, cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&l.done, cudaEventDisableTiming));
-        CU(cudaMalloc(&l.counter, kCounterBytes));
-        CU(cudaMalloc(&l.steal, (size_t)e->sm_count * 32 * kStealMaxResults * sizeof(StealResult)));
-    }
-    if (n == 0) return BGX_OK;
-    void *dq, *dc, *dm, *dl, *dv, *dn, *ds;
-    int rc;
-    if ((rc = lane_scratch(l, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = lane_scratch(l, 1, (size_t)n * 32, &dc))) return rc;
-    if ((rc = lane_scratch(l, 2, (size_t)n * 8, &dm))) return rc;
-    if ((rc = lane_scratch(l, 3, (size_t)n, &dl))) return rc;
-    if ((rc = lane_scratch(l, 4, (size_t)n * 4, &dv))) return rc;
-    if ((rc = lane_scratch(l, 5, (size_t)n * 4, &dn))) return rc;
-    if ((rc = lane_scratch(l, 6, (size_t)n * 4, &ds))) return rc;
-    // weights set on the engine's stream before this call are visible to the lane
-    CU(cudaEventRecord(e->ev_sync, e->stream));
-    CU(cudaStreamWaitEvent(l.stream, e->ev_sync, 0));
-    CU(cudaMemcpyAsync(dq, queries, (size_t)n * 32, cudaMemcpyHostToDevice, l.stream));
-    const SelectOut out = {chosen ? (int8_t *)dc : nullptr, moves ? (int8_t *)dm : nullptr, moves_len ? (int8_t *)dl : nullptr,
-                           value ? (float *)dv : nullptr, n_seq ? (int32_t *)dn : nullptr, n_scored ? (int32_t *)ds : nullptr};
-    void *region = nullptr;
-    if (n <= e->select_order_max && (rc = lane_scratch(l, 7, (size_t)n * kOrderBuckets * 4, &region))) return rc;
-    OrderPlan plan;
-    plan.region[0] = (int32_t *)region;
-    l.order_n = -1;
-    if ((rc = launch_select(e, l.stream, l.counter, l.steal, (const int8_t *)dq, n, epsilon, seed, out, plan, e->lane_grid))) return rc;
-    if (chosen) CU(cudaMemcpyAsync(chosen, dc, (size_t)n * 32, cudaMemcpyDeviceToHost, l.stream));
-    if (moves) CU(cudaMemcpyAsync(moves, dm, (size_t)n * 8, cudaMemcpyDeviceToHost, l.stream));
-    if (moves_len) CU(cudaMemcpyAsync(moves_len, dl, (size_t)n, cudaMemcpyDeviceToHost, l.stream));
-    if (value) CU(cudaMemcpyAsync(value, dv, (size_t)n * 4, cudaMemcpyDeviceToHost, l.stream));
-    if (n_seq) CU(cudaMemcpyAsync(n_seq, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, l.stream));
-    if (n_scored) CU(cudaMemcpyAsync(n_scored, ds, (size_t)n * 4, cudaMemcpyDeviceToHost, l.stream));
-    CU(cudaEventRecord(l.done, l.stream));
-    l.busy = true;
-    return BGX_OK;
-}
-
-static int play_ply(bgx_engine *e, int lane, const int8_t *records, int32_t *ply, int64_t *game_id, int64_t id_stride, int first_mover,
-                    int64_t n, float epsilon, uint64_t explore_seed, uint64_t dice_seed,
-                    int8_t *next_records, int8_t *winner, float *value, int32_t *n_seq, const char *who)
-{
-    NEED(lane >= 0 && lane < kLanes, "lane out of range");
-    NEED(records && next_records && n >= 0, "bad argument");
-    if (!e->have_weights) { set_error("%s: weights not set", who); return BGX_E_STATE; }
+    if (lane < 0 || lane >= kLanes) { set_error("%s: lane out of range", who); return BGX_E_INVALID; }
+    if (int rc = need_weights(e, who)) return rc;
     bgx_lane &l = e->lanes[lane];
     if (l.busy) { set_error("%s: lane %d has a batch in flight (bgx_lane_wait first)", who, lane); return BGX_E_STATE; }
     if (!l.stream) {
@@ -999,50 +973,72 @@ static int play_ply(bgx_engine *e, int lane, const int8_t *records, int32_t *ply
         CU(cudaMalloc(&l.counter, kCounterBytes));
         CU(cudaMalloc(&l.steal, (size_t)e->sm_count * 32 * kStealMaxResults * sizeof(StealResult)));
     }
-    if (n == 0) return BGX_OK;
-    void *dq, *dc, *dw, *dv, *dn, *dp = nullptr, *dg = nullptr, *r0 = nullptr, *r1 = nullptr;
-    int rc;
-    if ((rc = lane_scratch(l, 0, (size_t)n * 32, &dq))) return rc;
-    if ((rc = lane_scratch(l, 1, (size_t)n * 32, &dc))) return rc;
-    if ((rc = lane_scratch(l, 3, (size_t)n, &dw))) return rc;
-    if ((rc = lane_scratch(l, 4, (size_t)n * 4, &dv))) return rc;
-    if ((rc = lane_scratch(l, 5, (size_t)n * 4, &dn))) return rc;
-    if (ply && (rc = lane_scratch(l, 8, (size_t)n * 4, &dp))) return rc;
-    if (game_id && (rc = lane_scratch(l, 9, (size_t)n * 8, &dg))) return rc;
-    OrderPlan plan;
-    if (n <= e->select_order_max) {
-        const void *before[2] = {l.buf[7], l.buf[10]};
-        if ((rc = lane_scratch(l, 7, (size_t)n * kOrderBuckets * 4, &r0))) return rc;
-        if ((rc = lane_scratch(l, 10, (size_t)n * kOrderBuckets * 4, &r1))) return rc;
-        if (before[0] != l.buf[7] || before[1] != l.buf[10]) l.order_n = -1;      // reallocated: the stored queue is gone
-        plan.region[0] = (int32_t *)r0;
-        plan.region[1] = (int32_t *)r1;
-        plan.slot = l.order_slot;
-        plan.ready = l.order_n == n;           // the previous call on this lane sorted ITS outputs for us: if the caller's
-        plan.produce = true;                   // queries are something else the order is merely a poor one, never wrong
-    }
     CU(cudaEventRecord(e->ev_sync, e->stream));
     CU(cudaStreamWaitEvent(l.stream, e->ev_sync, 0));
-    CU(cudaMemcpyAsync(dq, records, (size_t)n * 32, cudaMemcpyHostToDevice, l.stream));
-    if (dp) CU(cudaMemcpyAsync(dp, ply, (size_t)n * 4, cudaMemcpyHostToDevice, l.stream));
-    if (dg) CU(cudaMemcpyAsync(dg, game_id, (size_t)n * 8, cudaMemcpyHostToDevice, l.stream));
-    const SelectOut out = {nullptr, nullptr, nullptr, value ? (float *)dv : nullptr, n_seq ? (int32_t *)dn : nullptr, nullptr};
-    AdvanceOut adv = {(int8_t *)dc, winner ? (int8_t *)dw : nullptr, (const int32_t *)dp, (const long long *)dg,
-                      (uint32_t)dice_seed, (uint32_t)(dice_seed >> 32), nullptr, nullptr,
-                      (long long)id_stride, first_mover, id_stride > 0 ? (int32_t *)dp : nullptr, id_stride > 0 ? (long long *)dg : nullptr};
-    if ((rc = launch_select(e, l.stream, l.counter, l.steal, (const int8_t *)dq, n, epsilon, explore_seed, out, plan, e->lane_grid, adv))) return rc;
-    if (plan.produce) { l.order_slot = 1 - plan.slot; l.order_n = n; }
-    CU(cudaMemcpyAsync(next_records, dc, (size_t)n * 32, cudaMemcpyDeviceToHost, l.stream));
-    if (winner) CU(cudaMemcpyAsync(winner, dw, (size_t)n, cudaMemcpyDeviceToHost, l.stream));
-    if (value) CU(cudaMemcpyAsync(value, dv, (size_t)n * 4, cudaMemcpyDeviceToHost, l.stream));
-    if (n_seq) CU(cudaMemcpyAsync(n_seq, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, l.stream));
-    if (id_stride > 0) {
-        CU(cudaMemcpyAsync(ply, dp, (size_t)n * 4, cudaMemcpyDeviceToHost, l.stream));
-        CU(cudaMemcpyAsync(game_id, dg, (size_t)n * 8, cudaMemcpyDeviceToHost, l.stream));
-    }
-    CU(cudaEventRecord(l.done, l.stream));
-    l.busy = true;
+    *out = &l;
     return BGX_OK;
+}
+
+// Asynchronous form of bgx_select_moves_host: the copies and the kernel are queued on lane `lane`'s own
+// stream and the call returns; bgx_lane_wait blocks until that lane's results are in the host buffers.
+// A few lanes in flight let the host advance one part of a population while the GPU plays the others.
+int bgx_select_moves_host_async(bgx_engine *e, int lane, const int8_t *queries, int64_t n, float epsilon, uint64_t seed,
+                                int8_t *chosen, int8_t *moves, int8_t *moves_len, float *value, int32_t *n_seq, int32_t *n_scored)
+{
+    USE(e);
+    NEED(queries && n >= 0, "bad argument");
+    bgx_lane *l;
+    if (int rc = lane_begin(e, lane, "bgx_select_moves_host_async", &l)) return rc;
+    if (n == 0) return BGX_OK;
+    OrderPlan plan;
+    if (n <= e->select_order_max) {
+        if (int rc = l->work.grow(kLaneOrder0, (size_t)n * kOrderBuckets * 4, &plan.region[0])) return rc;
+    }
+    l->order_n = -1;
+    Stage s(*l);
+    const int8_t *dq = s.in(queries, (size_t)n * 32);
+    const SelectOut out = {s.out(chosen, (size_t)n * 32), s.out(moves, (size_t)n * 8), s.out(moves_len, (size_t)n),
+                           s.out(value, (size_t)n * 4), s.out(n_seq, (size_t)n * 4), s.out(n_scored, (size_t)n * 4)};
+    if (s.rc) return s.rc;
+    return s.finish(launch_select(e, l->stream, l->counter, l->steal, dq, n, epsilon, seed, out, plan, e->lane_grid));
+}
+
+static int play_ply(bgx_engine *e, int lane, const int8_t *records, int32_t *ply, int64_t *game_id, int64_t id_stride, int first_mover,
+                    int64_t n, float epsilon, uint64_t explore_seed, uint64_t dice_seed,
+                    int8_t *next_records, int8_t *winner, float *value, int32_t *n_seq, const char *who)
+{
+    NEED(records && next_records && n >= 0, "bad argument");
+    bgx_lane *l;
+    if (int rc = lane_begin(e, lane, who, &l)) return rc;
+    if (n == 0) return BGX_OK;
+    OrderPlan plan;
+    if (n <= e->select_order_max) {
+        const void *before[2] = {l->work.buf[kLaneOrder0], l->work.buf[kLaneOrder1]};
+        int rc;
+        if ((rc = l->work.grow(kLaneOrder0, (size_t)n * kOrderBuckets * 4, &plan.region[0]))) return rc;
+        if ((rc = l->work.grow(kLaneOrder1, (size_t)n * kOrderBuckets * 4, &plan.region[1]))) return rc;
+        if (before[0] != plan.region[0] || before[1] != plan.region[1]) l->order_n = -1;   // reallocated: the stored queue is gone
+        plan.slot = l->order_slot;
+        plan.ready = l->order_n == n;          // the previous call on this lane sorted ITS outputs for us: if the caller's
+        plan.produce = true;                   // queries are something else the order is merely a poor one, never wrong
+    }
+    Stage s(*l);
+    const int8_t *dq = s.in(records, (size_t)n * 32);
+    int32_t *dp = s.in(ply, (size_t)n * 4);
+    long long *dg = s.in((long long *)game_id, (size_t)n * 8);
+    int8_t *dc = s.out(next_records, (size_t)n * 32);
+    int8_t *dw = s.out(winner, (size_t)n);
+    const SelectOut out = {nullptr, nullptr, nullptr, s.out(value, (size_t)n * 4), s.out(n_seq, (size_t)n * 4), nullptr};
+    if (id_stride > 0) {                       // restart mode: the kernel updates ply and game id in place
+        s.copy_back(ply, dp, (size_t)n * 4);
+        s.copy_back(game_id, dg, (size_t)n * 8);
+    }
+    if (s.rc) return s.rc;
+    AdvanceOut adv = {dc, dw, dp, dg, (uint32_t)dice_seed, (uint32_t)(dice_seed >> 32), nullptr, nullptr,
+                      (long long)id_stride, first_mover, id_stride > 0 ? dp : nullptr, id_stride > 0 ? dg : nullptr};
+    if (int rc = launch_select(e, l->stream, l->counter, l->steal, dq, n, epsilon, explore_seed, out, plan, e->lane_grid, adv)) return rc;
+    if (plan.produce) { l->order_slot = 1 - plan.slot; l->order_n = n; }
+    return s.finish();
 }
 
 // One iteration of play_game's loop (train.py:103-121) for n games through host buffers, asynchronous:
@@ -1150,7 +1146,7 @@ int bgx_selfplay_next_round(bgx_engine *e)
 static int run_selfplay(bgx_engine *e, int n_plies, int round_mode, float epsilon, bgx_stats *out)
 {
     if (e->n_slots == 0) { set_error("self-play: call bgx_selfplay_init first"); return BGX_E_STATE; }
-    if (!e->have_weights) { set_error("self-play: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "self-play")) return rc;
     SelfplayParams p;
     p.slots = e->slots; p.ply = e->ply; p.game_id = e->game_id;
     p.traj_pre = e->traj_pre; p.traj_chosen = e->traj_chosen;
@@ -1162,13 +1158,12 @@ static int run_selfplay(bgx_engine *e, int n_plies, int round_mode, float epsilo
     CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
     CU(cudaMemsetAsync(e->stats, 0, 16 * sizeof(unsigned long long), e->stream));
     tick(e);
-#define BGX_LAUNCH_SELFPLAY(W, S, X) k_selfplay<W, S, X><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, e->fixed, e->flat, e->steal)
-    const bool ex = epsilon > 0.f;
-    if (e->selfplay_warps == 16) { if (ex) BGX_LAUNCH_SELFPLAY(16, 109, true); else BGX_LAUNCH_SELFPLAY(16, 109, false); }
-    else if (e->selfplay_warps == 20) { if (ex) BGX_LAUNCH_SELFPLAY(20, 86, true); else BGX_LAUNCH_SELFPLAY(20, 86, false); }
-    else if (e->selfplay_warps == 24) { if (ex) BGX_LAUNCH_SELFPLAY(24, 72, true); else BGX_LAUNCH_SELFPLAY(24, 72, false); }
-    else { if (ex) BGX_LAUNCH_SELFPLAY(32, 53, true); else BGX_LAUNCH_SELFPLAY(32, 53, false); }
-#undef BGX_LAUNCH_SELFPLAY
+    PlyConfigs::dispatch(e->selfplay_warps, [&](auto c) {
+        constexpr int W = decltype(c)::kWarps, S = decltype(c)::kSets;
+        dispatch_explore(epsilon > 0.f, [&](auto x) {
+            k_selfplay<W, S, decltype(x)::value><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, e->fixed, e->flat, e->steal);
+        });
+    });
     tock(e);
     e->launches++;
     CU(cudaGetLastError());
@@ -1245,14 +1240,10 @@ int bgx_selfplay_sample_host(bgx_engine *e, int32_t per_game, uint64_t seed, int
 {
     USE(e);
     NEED(records && per_game > 0, "bad argument");
-    void *d;
-    int rc;
-    const size_t bytes = (size_t)e->n_slots * per_game * 32;
-    if ((rc = scratch(e, 0, bytes, &d))) return rc;
-    if ((rc = bgx_selfplay_sample(e, per_game, seed, (int8_t *)d))) return rc;
-    CU(cudaMemcpyAsync(records, d, bytes, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return BGX_OK;
+    Stage s(e);
+    int8_t *d = s.out(records, (size_t)e->n_slots * per_game * 32);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_selfplay_sample(e, per_game, seed, d));
 }
 
 // ------------------------------------------------------------------------ TD(lambda)
@@ -1333,7 +1324,7 @@ static int td_replay_population(bgx_engine *e, double lr, double lambda, long lo
 {
     NEED(delta_dev, "null delta buffer");
     if (e->n_slots == 0 || !e->traj_pre) { set_error("TD replay: needs a population created with traj_cap > 0"); return BGX_E_STATE; }
-    if (!e->have_weights) { set_error("TD replay: weights not set"); return BGX_E_STATE; }
+    if (int rc = need_weights(e, "TD replay")) return rc;
     return launch_td(e, e->traj_pre, e->slots, e->ply, e->n_slots, e->traj_cap, lr, lambda, episode_first, delta_dev, nullptr, nullptr, out);
 }
 
@@ -1381,31 +1372,21 @@ int bgx_td_replay_host(bgx_engine *e, const int8_t *records, int32_t T, int play
 {
     USE(e);
     NEED(records && T > 0 && T <= kTdMaxSteps && new_W1 && new_b1 && new_w2 && new_b2, "bad argument (1 <= T <= BGX_TD_MAX_STEPS)");
-    if (!e->have_weights) { set_error("bgx_td_replay_host: weights not set"); return BGX_E_STATE; }
-    void *dtraj, *dslot, *dply, *dfinal, *dsq;
-    int rc;
-    if ((rc = scratch(e, 0, (size_t)T * 32, &dtraj))) return rc;
-    if ((rc = scratch(e, 1, 32, &dslot))) return rc;
-    if ((rc = scratch(e, 2, 4, &dply))) return rc;
-    if ((rc = scratch(e, 9, BGX_NPARAMS_PADDED * sizeof(float), &dfinal))) return rc;
-    if ((rc = scratch(e, 10, (size_t)T * 8, &dsq))) return rc;
+    if (int rc = need_weights(e, "bgx_td_replay_host")) return rc;
     int8_t slot[32] = {0};
     slot[31] = player1_won ? kP1Won : kP2Won;
-    CU(cudaMemcpyAsync(dtraj, records, (size_t)T * 32, cudaMemcpyHostToDevice, e->stream));
-    CU(cudaMemcpyAsync(dslot, slot, 32, cudaMemcpyHostToDevice, e->stream));
-    CU(cudaMemcpyAsync(dply, &T, 4, cudaMemcpyHostToDevice, e->stream));
-    CU(cudaMemsetAsync(dsq, 0, (size_t)T * 8, e->stream));
-    if ((rc = launch_td(e, (const int8_t *)dtraj, (const int8_t *)dslot, (const int32_t *)dply, 1, T, lr, lambda, -1,
-                        nullptr, (float *)dfinal, (double *)dsq, nullptr)))
-        return rc;
     std::vector<float> flat(BGX_NPARAMS_PADDED);
-    CU(cudaMemcpyAsync(flat.data(), dfinal, flat.size() * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
-    if (sq_errors && T > 1) CU(cudaMemcpyAsync(sq_errors, dsq, (size_t)(T - 1) * 8, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    std::memcpy(new_W1, flat.data(), kTableFloats * sizeof(float));
-    std::memcpy(new_b1, flat.data() + kTableFloats, kHidden * sizeof(float));
-    std::memcpy(new_w2, flat.data() + kTableFloats + kHidden, kHidden * sizeof(float));
-    new_b2[0] = flat[kTableFloats + 2 * kHidden];
+    Stage s(e);
+    const int8_t *dtraj = s.in(records, (size_t)T * 32);
+    const int8_t *dslot = s.in(slot, 32);
+    const int32_t *dply = s.in(&T, 4);
+    float *dfinal = s.out(flat.data(), flat.size() * sizeof(float));
+    double *dsq = s.take<double>((size_t)T * 8);
+    if (s.rc) return s.rc;
+    if (sq_errors && T > 1) s.copy_back(sq_errors, dsq, (size_t)(T - 1) * 8);
+    CU(cudaMemsetAsync(dsq, 0, (size_t)T * 8, e->stream));
+    if (int rc = s.finish(launch_td(e, dtraj, dslot, dply, 1, T, lr, lambda, -1, nullptr, dfinal, dsq, nullptr))) return rc;
+    unpack_weights(flat.data(), new_W1, new_b1, new_w2, new_b2);
     return BGX_OK;
 }
 

@@ -24,6 +24,30 @@ constexpr int ply_smem()
 {
     return kFixedBytes + kWarps * (int)sizeof(PlyScratch<kSets>) + (int)sizeof(StealShared<kWarps>) + kWarps * (int)sizeof(WarpSeat) + 16;
 }
+
+// the launch configurations of the fused ply kernels (k_select, k_selfplay, k_rollout): warps per CTA and the cache sets per
+// warp that fill the shared memory at that width.  Each kernel is instantiated once per entry.
+template <int W, int S>
+struct PlyConfig {
+    static constexpr int kWarps = W, kSets = S, kSmem = ply_smem<W, S>();
+};
+template <typename... C>
+struct PlyConfigList {
+    static constexpr bool has(long long warps) { return ((warps == C::kWarps) || ...); }
+    static constexpr bool fits(int smem_bytes) { return ((C::kSmem <= smem_bytes) && ...); }
+    // f(config) for every configuration, stopping at the first non-zero result, which is returned
+    template <typename F>
+    static int each(F &&f)
+    {
+        int rc = 0;
+        ((rc = rc ? rc : f(C{})), ...);
+        return rc;
+    }
+    // f(config) for the configuration with `warps` warps per CTA
+    template <typename F>
+    static void dispatch(int warps, F &&f) { ((warps == C::kWarps ? f(C{}) : void()), ...); }
+};
+using PlyConfigs = PlyConfigList<PlyConfig<16, 109>, PlyConfig<20, 86>, PlyConfig<24, 72>, PlyConfig<32, 53>>;
 constexpr int kEvalSmem = kFixedBytes + 16;            // k_evaluate: table + barrier
 
 // exact-dedup table of the summary kernel: per warp, in global memory (L2 resident)
