@@ -68,6 +68,8 @@ _SIGNATURES = {
     "bgx_select_moves_2ply_host": (C.c_int, [_vp, _vp, _i64, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_rollout": (C.c_int, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_uint64, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_rollout_host": (C.c_int, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_uint64, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "bgx_rollout_vr": (C.c_int, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_uint64, C.c_int, C.c_int32] + [_vp] * 9),
+    "bgx_rollout_vr_host": (C.c_int, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_uint64, C.c_int, C.c_int32] + [_vp] * 9),
     "bgx_select_moves_host_async":(C.c_int, [_vp, C.c_int, _vp, _i64, C.c_float, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bgx_play_ply_host_async": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _i64, C.c_float, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),
     "bgx_play_ply_restart_host_async": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _i64, C.c_int, _i64, C.c_float, C.c_uint64, C.c_uint64, _vp, _vp, _vp, _vp]),

@@ -197,16 +197,20 @@ class TDLGammonModel(nn.Module):
             result.append(seq)
         return result
 
-    def rollout_batch(self, games, trials=1296, max_plies=0, seed=0x5EED2026, device=0):
+    def rollout_batch(self, games, trials=1296, max_plies=0, seed=0x5EED2026, device=0, vr_plies=0):
         """Rollouts of compat Game objects (BatchEngine.rollout_host, DESIGN 7d): `trials` greedy games from each game's
         position with its player on roll (the dice are ignored), stratified over the first roll when trials is a multiple of 36,
         cut after `max_plies` plies (0: played to the end).  The games are not modified.
         -> dict(p1_win f64[n] = P(PLAYER1 wins), std_err f64[n], outcomes f64[n, 6] = fractions of PLAYER1 single / gammon /
-        backgammon and PLAYER2 single / gammon / backgammon wins)"""
+        backgammon and PLAYER2 single / gammon / backgammon wins).  vr_plies > 0 (DESIGN 7e) adds vr_p1_win and vr_std_err, the
+        luck-adjusted estimate over the first vr_plies plies of each trial and its standard error."""
         trials = int(trials)
         out = self.engine(device).rollout_host(_game_records(games), trials, max_plies=max_plies, seed=seed,
-                                               stratify=trials % 36 == 0)
-        return {"p1_win": out["mean"], "std_err": out["std_err"], "outcomes": out["counts"][:, :6] / float(trials)}
+                                               stratify=trials % 36 == 0, vr_plies=vr_plies)
+        r = {"p1_win": out["mean"], "std_err": out["std_err"], "outcomes": out["counts"][:, :6] / float(trials)}
+        if vr_plies:
+            r["vr_p1_win"], r["vr_std_err"] = out["vr_mean"], out["vr_std_err"]
+        return r
 
 
 def _game_records(games):

@@ -289,24 +289,37 @@ class BatchEngine {
         d["chosen"] = chosen; d["moves"] = moves; d["moves_len"] = len; d["value"] = value; d["n_candidates"] = n_cand; d["n_expanded"] = n_exp;
         return d;
     }
-    py::dict rollout(I8 q, int32_t trials, int32_t max_plies, uint64_t seed, bool stratify, bool per_trial)
+    py::dict rollout(I8 q, int32_t trials, int32_t max_plies, uint64_t seed, bool stratify, bool per_trial, int32_t vr_plies)
     {
         int64_t n = rows(q);
         const py::ssize_t T = per_trial && trials > 0 ? trials : 0;
-        py::array_t<double> mean(n), std_err(n);
+        py::array_t<double> mean(n), std_err(n), vr_mean(n), vr_std_err(n);
         py::array_t<int64_t> counts({(py::ssize_t)n, (py::ssize_t)8});
         py::array_t<float> value({(py::ssize_t)n, T});
         py::array_t<int8_t> outcome({(py::ssize_t)n, T});
         py::array_t<int32_t> plies({(py::ssize_t)n, T});
+        py::array_t<double> luck({(py::ssize_t)n, vr_plies ? T : 0});
         {
             py::gil_scoped_release nogil;
-            Game::check(bgx_rollout_host(e_, q.data(), n, trials, max_plies, seed, stratify ? BGX_ROLLOUT_STRATIFY : 0, mean.mutable_data(),
-                                         std_err.mutable_data(), counts.mutable_data(), per_trial ? value.mutable_data() : nullptr,
-                                         per_trial ? outcome.mutable_data() : nullptr, per_trial ? plies.mutable_data() : nullptr));
+            const int flags = stratify ? BGX_ROLLOUT_STRATIFY : 0;
+            float *v = per_trial ? value.mutable_data() : nullptr;
+            int8_t *o = per_trial ? outcome.mutable_data() : nullptr;
+            int32_t *p = per_trial ? plies.mutable_data() : nullptr;
+            if (vr_plies)
+                Game::check(bgx_rollout_vr_host(e_, q.data(), n, trials, max_plies, seed, flags, vr_plies, mean.mutable_data(), std_err.mutable_data(),
+                                                counts.mutable_data(), v, o, p, vr_mean.mutable_data(), vr_std_err.mutable_data(),
+                                                per_trial ? luck.mutable_data() : nullptr));
+            else
+                Game::check(bgx_rollout_host(e_, q.data(), n, trials, max_plies, seed, flags, mean.mutable_data(), std_err.mutable_data(),
+                                             counts.mutable_data(), v, o, p));
         }
         py::dict d;
         d["mean"] = mean; d["std_err"] = std_err; d["counts"] = counts;
         if (per_trial) { d["trial_value"] = value; d["trial_outcome"] = outcome; d["trial_plies"] = plies; }
+        if (vr_plies) {
+            d["vr_mean"] = vr_mean; d["vr_std_err"] = vr_std_err;
+            if (per_trial) d["trial_luck"] = luck;
+        }
         return d;
     }
     py::array_t<float> encode(I8 q)
@@ -477,7 +490,7 @@ PYBIND11_MODULE(backgammon_env, m)
         .def("make_moves", &BatchEngine::make_moves, py::arg("queries"), py::arg("epsilon") = 0.0f, py::arg("seed") = 0)
         .def("make_moves_2ply", &BatchEngine::make_moves_2ply, py::arg("queries"), py::arg("max_candidates") = 0)
         .def("rollout", &BatchEngine::rollout, py::arg("positions"), py::arg("trials"), py::arg("max_plies") = 0,
-             py::arg("seed") = 0x5EED2026ull, py::arg("stratify") = true, py::arg("per_trial") = false)
+             py::arg("seed") = 0x5EED2026ull, py::arg("stratify") = true, py::arg("per_trial") = false, py::arg("vr_plies") = 0)
         .def("encode", &BatchEngine::encode)
         .def("evaluate", &BatchEngine::evaluate)
         .def("get_weights", &BatchEngine::get_weights)

@@ -68,12 +68,13 @@ enum Work {
     kTpRecords, kTpMoves, kTpMovesLen, kTpValue, kTpExpand, kTpE2, kTpList,
     // per chunk of replies: records, values, sorted queue
     kTpReplies, kTpReplyValue, kTpReplyOrder,
-    // bgx_rollout: the per-trial results of a chunk the caller did not ask for
-    kRolloutValue, kRolloutOutcome, kRolloutPlies,
+    // bgx_rollout / bgx_rollout_vr: the per-trial results of a chunk the caller did not ask for
+    kRolloutValue, kRolloutOutcome, kRolloutPlies, kRolloutLuck,
+    kRolloutRolls, kRolloutZlist,                    // k_rollout_vr: per warp, the roll values of its ply and the 21-roll walks' stash
     kWorkBufs
 };
 enum LaneWork { kLaneOrder0, kLaneOrder1, kLaneWorkBufs };   // a lane's sorted queues: the one read, the one written for the next call
-constexpr int kStageBufs = 7;                    // the most host arrays one *_host call stages
+constexpr int kStageBufs = 10;                   // the most host arrays one *_host call stages (bgx_rollout_vr_host)
 
 // an asynchronous lane of the batched make_move path: its own stream, work-queue counter,
 // sharing buffer and staging buffers, so that two batches can be in flight at once
@@ -282,6 +283,7 @@ static int create_into(bgx_engine *e, int device, const cudaDeviceProp &prop)
         CU(cudaFuncSetAttribute(k_selfplay<W, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
         CU(cudaFuncSetAttribute(k_selfplay<W, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
         CU(cudaFuncSetAttribute(k_rollout<W, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
+        CU(cudaFuncSetAttribute(k_rollout_vr<W, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.kSmem));
         return BGX_OK;
     });
     if (rc) return rc;
@@ -323,7 +325,7 @@ int bgx_create(int device, bgx_engine **out)
 //   "select_lane_grid"                 CTAs of a launch on an asynchronous lane (0: one per SM; default: half the SMs)
 //   "select_order_max"                 largest batch that gets a sorted queue
 //   "select_urgent_min" / "select_giant_min" / "select_urgent_from_pct"   when a CTA helps a published double
-//   "rollout_warps"                    warps per CTA of k_rollout: 16, 20, 24 or 32
+//   "rollout_warps"                    warps per CTA of k_rollout and k_rollout_vr: 16, 20, 24 or 32
 //   "rollout_chunk"                    trials (games) per k_rollout launch, rounded down to whole positions (0: 2^24)
 int bgx_set_option(bgx_engine *e, const char *key, int64_t value)
 {
@@ -888,31 +890,36 @@ static int rollout_args(int64_t n, int32_t trials, int32_t max_plies, int flags,
     return BGX_OK;
 }
 
-int bgx_rollout(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
-                double *mean, double *std_err, int64_t *counts, float *trial_value, int8_t *trial_outcome, int32_t *trial_plies)
+// bgx_rollout (vr_plies < 0: k_rollout) and bgx_rollout_vr (k_rollout_vr), arguments checked
+static int rollout_run(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                       int32_t vr_plies, double *mean, double *std_err, int64_t *counts, float *trial_value, int8_t *trial_outcome,
+                       int32_t *trial_plies, double *vr_mean, double *vr_std_err, double *trial_luck)
 {
-    USE(e);
-    if (int rc = rollout_args(n, trials, max_plies, flags, "bgx_rollout")) return rc;
-    NEED(positions || n == 0, "null positions");
-    if (int rc = need_weights(e, "bgx_rollout")) return rc;
-    if (n == 0) return BGX_OK;
     // chunks of whole positions; the per-trial results of a chunk go to the caller's arrays or to engine work buffers
     const long long chunk = e->rollout_chunk > 0 ? e->rollout_chunk : kRolloutChunk;
     const long long per_launch = std::max<long long>(1, chunk / trials);
     const long long items_cap = std::min<long long>(n, per_launch) * trials;
+    const bool vr = vr_plies >= 0;
     float *sv = nullptr;
     int8_t *so = nullptr;
     int32_t *sp = nullptr;
+    double *sl = nullptr;
     int rc;
     if (!trial_value && (rc = e->work.grow(kRolloutValue, (size_t)items_cap * 4, &sv))) return rc;
     if (!trial_outcome && (rc = e->work.grow(kRolloutOutcome, (size_t)items_cap, &so))) return rc;
     if (!trial_plies && (rc = e->work.grow(kRolloutPlies, (size_t)items_cap * 4, &sp))) return rc;
+    if (vr && !trial_luck && (rc = e->work.grow(kRolloutLuck, (size_t)items_cap * 8, &sl))) return rc;
+    float *rolls = nullptr;
+    int4 *zlist = nullptr;
+    if (vr && (rc = e->work.grow(kRolloutRolls, (size_t)game_grid(e) * 32 * 32 * 4, &rolls))) return rc;
+    if (vr && (rc = e->work.grow(kRolloutZlist, (size_t)game_grid(e) * 32 * 32 * sizeof(int4), &zlist))) return rc;
     RolloutParams p;
     p.trials = trials;
     p.cap = max_plies > 0 ? max_plies : BGX_ROLLOUT_MAX_PLIES;
     p.stratify = (flags & BGX_ROLLOUT_STRATIFY) ? 1 : 0;
     p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
     p.counter = e->counter; p.zstash = e->zstash;
+    RolloutVR r = {vr_plies, nullptr, rolls, zlist};
     tick(e);
     for (long long q0 = 0; q0 < n; q0 += per_launch) {
         const long long np = std::min<long long>(n - q0, per_launch);
@@ -922,20 +929,39 @@ int bgx_rollout(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trial
         p.value = trial_value ? trial_value + at : sv;
         p.outcome = trial_outcome ? trial_outcome + at : so;
         p.plies = trial_plies ? trial_plies + at : sp;
+        r.luck = trial_luck ? trial_luck + at : sl;
         CU(cudaMemsetAsync(e->counter, 0, sizeof(unsigned long long), e->stream));
         PlyConfigs::dispatch(e->rollout_warps, [&](auto c) {
             constexpr int W = decltype(c)::kWarps, S = decltype(c)::kSets;
-            k_rollout<W, S><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, e->fixed, e->steal);
+            if (vr) k_rollout_vr<W, S><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, r, e->fixed, e->steal);
+            else k_rollout<W, S><<<game_grid(e), W * 32, ply_smem<W, S>(), e->stream>>>(p, e->fixed, e->steal);
         });
+        const unsigned grid = (unsigned)((np + 127) / 128);
         if (mean || std_err || counts)
-            k_rollout_reduce<<<(unsigned)((np + 127) / 128), 128, 0, e->stream>>>(p.value, p.outcome, p.plies, np, trials, mean ? mean + q0 : nullptr,
-                                                                              std_err ? std_err + q0 : nullptr,
-                                                                              counts ? (long long *)counts + q0 * 8 : nullptr);
+            k_rollout_reduce<<<grid, 128, 0, e->stream>>>(p.value, p.outcome, p.plies, np, trials, mean ? mean + q0 : nullptr,
+                                                          std_err ? std_err + q0 : nullptr, counts ? (long long *)counts + q0 * 8 : nullptr);
         e->launches += 2;
+        if (vr_mean || vr_std_err) {
+            k_rollout_vr_reduce<<<grid, 128, 0, e->stream>>>(p.value, r.luck, np, trials, vr_mean ? vr_mean + q0 : nullptr,
+                                                             vr_std_err ? vr_std_err + q0 : nullptr);
+            e->launches++;
+        }
         CU(cudaGetLastError());
     }
     tock(e);
     return BGX_OK;
+}
+
+int bgx_rollout(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                double *mean, double *std_err, int64_t *counts, float *trial_value, int8_t *trial_outcome, int32_t *trial_plies)
+{
+    USE(e);
+    if (int rc = rollout_args(n, trials, max_plies, flags, "bgx_rollout")) return rc;
+    NEED(positions || n == 0, "null positions");
+    if (int rc = need_weights(e, "bgx_rollout")) return rc;
+    if (n == 0) return BGX_OK;
+    return rollout_run(e, positions, n, trials, max_plies, seed, flags, -1, mean, std_err, counts, trial_value, trial_outcome, trial_plies,
+                       nullptr, nullptr, nullptr);
 }
 
 int bgx_rollout_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
@@ -957,6 +983,53 @@ int bgx_rollout_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t 
     int32_t *dp = s.out(trial_plies, items * 4);
     if (s.rc) return s.rc;
     return s.finish(bgx_rollout(e, dq, n, trials, max_plies, seed, flags, dm, ds, dc, dv, dout, dp));
+}
+
+// ------------------------------------------------------------------------ variance-reduced rollouts (DESIGN 7e)
+
+static int rollout_vr_args(int64_t n, int32_t trials, int32_t max_plies, int flags, int32_t vr_plies, const char *who)
+{
+    if (int rc = rollout_args(n, trials, max_plies, flags, who)) return rc;
+    if (vr_plies < 0 || vr_plies > BGX_ROLLOUT_MAX_PLIES) { set_error("%s: vr_plies must be 0 .. %d", who, BGX_ROLLOUT_MAX_PLIES); return BGX_E_INVALID; }
+    return BGX_OK;
+}
+
+int bgx_rollout_vr(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                   int32_t vr_plies, double *mean, double *std_err, int64_t *counts, float *trial_value, int8_t *trial_outcome,
+                   int32_t *trial_plies, double *vr_mean, double *vr_std_err, double *trial_luck)
+{
+    USE(e);
+    if (int rc = rollout_vr_args(n, trials, max_plies, flags, vr_plies, "bgx_rollout_vr")) return rc;
+    NEED(positions || n == 0, "null positions");
+    if (int rc = need_weights(e, "bgx_rollout_vr")) return rc;
+    if (n == 0) return BGX_OK;
+    return rollout_run(e, positions, n, trials, max_plies, seed, flags, vr_plies, mean, std_err, counts, trial_value, trial_outcome,
+                       trial_plies, vr_mean, vr_std_err, trial_luck);
+}
+
+int bgx_rollout_vr_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                        int32_t vr_plies, double *mean, double *std_err, int64_t *counts, float *trial_value, int8_t *trial_outcome,
+                        int32_t *trial_plies, double *vr_mean, double *vr_std_err, double *trial_luck)
+{
+    USE(e);
+    if (int rc = rollout_vr_args(n, trials, max_plies, flags, vr_plies, "bgx_rollout_vr_host")) return rc;
+    NEED(positions || n == 0, "null positions");
+    if (int rc = need_weights(e, "bgx_rollout_vr_host")) return rc;
+    if (n == 0) return BGX_OK;
+    const size_t items = (size_t)n * trials;
+    Stage s(e);
+    const int8_t *dq = s.in(positions, (size_t)n * 32);
+    double *dm = s.out(mean, (size_t)n * 8);
+    double *ds = s.out(std_err, (size_t)n * 8);
+    int64_t *dc = s.out(counts, (size_t)n * 64);
+    float *dv = s.out(trial_value, items * 4);
+    int8_t *dout = s.out(trial_outcome, items);
+    int32_t *dp = s.out(trial_plies, items * 4);
+    double *dvm = s.out(vr_mean, (size_t)n * 8);
+    double *dvs = s.out(vr_std_err, (size_t)n * 8);
+    double *dl = s.out(trial_luck, items * 8);
+    if (s.rc) return s.rc;
+    return s.finish(bgx_rollout_vr(e, dq, n, trials, max_plies, seed, flags, vr_plies, dm, ds, dc, dv, dout, dp, dvm, dvs, dl));
 }
 
 // the start of a call on lane `lane`: the lane is free, its stream and buffers exist, and its stream waits for the work

@@ -3,11 +3,16 @@
 //                      from the position to its end or its truncation ply with the fused greedy ply (choose_ply_fast, the root-stash
 //                      carry, big doubles shared inside the CTA) and writes x_t, the outcome class and the ply count at index i
 //   k_rollout_reduce   one thread per position: mean, standard error and counts, float64, sequentially in trial order
+//   k_rollout_vr       k_rollout with luck-based variance reduction (DESIGN 7e): the same play; at each of the first vr_plies plies
+//                      of a trial the seated warp also walks the mover's 21 rolls, and adds the luck of the roll played (its value
+//                      minus the 21-roll expectation, float64) to the trial's luck at index i
+//   k_rollout_vr_reduce  one thread per position: mean and standard error of x_t - luck_t, as k_rollout_reduce forms them
 // Dice are a function of the trial index only (common random numbers), the values are the fixed-point evaluator's (pure functions
 // of the query, bgx_ply.cuh) and every trial's result lands at its own index: the outputs depend on nothing but
-// (position, mover, trials, max_plies, seed, flags, weights).
+// (position, mover, trials, max_plies, seed, flags, weights) (and vr_plies).
 #pragma once
 #include "bgx_kernels.cuh"
+#include "bgx_twoply.cuh"
 
 namespace bgx {
 
@@ -26,6 +31,15 @@ struct RolloutParams {
     int4 *zstash;             // [CTA][warp][32] (greedy_ply's root-stash carry)
 };
 
+// the variance reduction of k_rollout_vr
+struct RolloutVR {
+    int plies;                // plies k < plies of a trial are valued under all 21 rolls
+    double *luck;             // [n_items] the trial's summed luck, accumulated in ply order
+    float *rolls;             // [CTA][warp][32] the seated ply's roll values: lane r < 21 L(roll r), lane 31 V(position, mover)
+    int4 *zlist;              // [CTA][warp][32] the root stash of the 21-roll walks: written, never read, so that the trial's own
+                              // stash keeps the root for the played walk (a null stash instead spills at 20 warps)
+};
+
 // outcome class of a finished game, from the final board alone.  The loser is gammoned if it has borne nothing off, backgammoned
 // if it also has a checker on the bar or in the winner's home board (PLAYER1 bears off past index 23: its home is 18..23,
 // PLAYER2's is 0..5; bars are lanes 24 + player, counts positive, PLAYER1's checkers positive on the points)
@@ -39,9 +53,9 @@ __device__ __forceinline__ int outcome_class(int v, int lane, int winner)
     return winner == 0 ? cls : 3 + cls;
 }
 
-template <int kWarps, int kSets>
-__global__ void __launch_bounds__(kWarps * 32, 1)
-k_rollout(RolloutParams p, const int32_t *__restrict__ Ti, StealResult *__restrict__ steal)
+// the loop of k_rollout (kVR = false) and k_rollout_vr
+template <int kWarps, int kSets, bool kVR>
+__device__ __forceinline__ void rollout_loop(RolloutParams p, RolloutVR vr, const int32_t *__restrict__ Ti, StealResult *__restrict__ steal)
 {
     extern __shared__ __align__(128) unsigned char smem[];
     const PlySmem<kWarps, kSets> sm(smem);
@@ -57,7 +71,9 @@ k_rollout(RolloutParams p, const int32_t *__restrict__ Ti, StealResult *__restri
                            p.counter, (unsigned long long)(p.n_items - p.n_items / 4), 8, kGiantMinChildren};
     bool helping = false, seated = false;
     int v = 0, dice = 0;                                // dice: d1 | d2 << 4 of ply dice_base + lane of the trial
-    WarpSeat &S = sm.seat[warp];                        // slot = work item, gid = trial index, ply = plies played so far
+    // slot = work item, gid = trial index, ply = plies played so far; kVR: step = the seated ply's walk (roll r < 21 of the
+    // list, 21 the roll played), status = the played roll's list index | 32 if its list walk is the played walk (d1 >= d2)
+    WarpSeat &S = sm.seat[warp];
     int4 *const zmine = p.zstash + ((size_t)blockIdx.x * kWarps + warp) * 32 + lane;
     // one iteration = one ply: of the trial this warp is seated at, or of a sub-tree taken from a neighbour (k_selfplay's loop)
     for (;;) {
@@ -89,6 +105,7 @@ k_rollout(RolloutParams p, const int32_t *__restrict__ Ti, StealResult *__restri
                     const int winner = off1 == 15 ? 0 : 1;
                     const int cls = outcome_class(v, lane, winner);
                     if (lane == 0) { p.value[i] = winner == 0 ? 1.f : 0.f; p.outcome[i] = (int8_t)cls; p.plies[i] = 0; }
+                    if (kVR && lane == 0) vr.luck[i] = 0.0;
                     __syncwarp();
                     continue;
                 }
@@ -100,6 +117,7 @@ k_rollout(RolloutParams p, const int32_t *__restrict__ Ti, StealResult *__restri
                     S.ply = 0;
                     S.carry = 0;
                     S.dice_base = -1;
+                    if (kVR) { S.step = 0; vr.luck[i] = 0.0; }
                 }
                 __syncwarp();
                 seated = true;
@@ -129,12 +147,58 @@ k_rollout(RolloutParams p, const int32_t *__restrict__ Ti, StealResult *__restri
         // what the walk branches on, as values ptxas can PROVE warp-uniform (see k_selfplay)
         d1 = __shfl_sync(kFull, d1, 0); d2 = __shfl_sync(kFull, d2, 0);
         mover = __shfl_sync(kFull, mover, 0); only = __shfl_sync(kFull, only, 0);
+        bool listed = false;                            // kVR: a walk of the 21-roll list: its own stash, no carry
+        if constexpr (kVR) {
+            // A VR ply walks the list's rolls in order, then the roll played, last so that it carries the root stash as k_rollout's
+            // ply does.  When d1 >= d2 the played walk is also the list's walk of that roll, which is then not walked twice.
+            const int step = __shfl_sync(kFull, only == 0 && S.ply < vr.plies ? S.step : -1, 0);
+            if (step >= 0) {
+                if (step == 0) {                        // once per ply: the value of a blocked roll
+                    const float V = ev.finish(ev.preactivation(root, lane, mover), lane);
+                    if (lane == 31) vr.rolls[((size_t)blockIdx.x * kWarps + warp) * 32 + lane] = V;
+                }
+                const int hi = d1 > d2 ? d1 : d2, lo = d1 + d2 - hi;
+                const int actual = hi * (hi - 1) / 2 + lo - 1;
+                const int walk = step == actual && d1 >= d2 ? step + 1 : step;
+                if (lane == 0) { S.step = walk; S.status = actual | (d1 >= d2 ? 32 : 0); }
+                __syncwarp();
+                if (walk < kRolls) {
+                    d1 = kRollA[walk]; d2 = kRollB[walk];
+                    listed = true;
+                }
+            }
+        }
         const Choice c = choose_ply_fast<kSets, false>(root, lane, mover, d1, d2, ev, cache, false, 0u, only ? only : kFull,
-                                                       only ? nullptr : &mine, only ? nullptr : zmine,
-                                                       only == 0 && S.carry != 0);
+                                                       only ? nullptr : &mine,
+                                                       only ? nullptr : (kVR && listed ? vr.zlist + ((size_t)blockIdx.x * kWarps + warp) * 32 + lane
+                                                                                       : zmine),
+                                                       only == 0 && !listed && S.carry != 0);
         if (only) {
             deliver_child<kWarps>(sm.share, cta_results, vw, only, c, lane);
             continue;
+        }
+        if constexpr (kVR) {
+            const int walk = __shfl_sync(kFull, S.ply < vr.plies ? S.step : -1, 0);
+            if (walk >= 0) {
+                float *const rolls = vr.rolls + ((size_t)blockIdx.x * kWarps + warp) * 32;
+                const float Lw = c.any ? c.value : rolls[31];                     // two-ply's reply rule
+                if (walk < kRolls) {                    // a list walk: keep its value, play nothing
+                    if (lane == walk) rolls[lane] = Lw;
+                    if (lane == 0) S.step = walk + 1;
+                    __syncwarp();
+                    continue;
+                }
+                const int st = __shfl_sync(kFull, S.status, 0), actual = st & 31;
+                if ((st & 32) && lane == actual) rolls[lane] = Lw;
+                __syncwarp();
+                const float L = rolls[lane];
+                // E in two-ply's order and arithmetic (k_twoply_reduce), not rounded; luck = L(played) - E, summed in ply order
+                const double term = lane < kRolls ? (kRollA[lane] == kRollB[lane] ? 1.0 : 2.0) * (double)L : 0.0;
+                double acc = 0.0;
+                for (int r = 0; r < kRolls; r++) acc = __dadd_rn(acc, __shfl_sync(kFull, term, r));
+                const double luck = __dadd_rn((double)__shfl_sync(kFull, L, actual), -(acc / 36.0));
+                if (lane == 0) { vr.luck[S.slot] = __dadd_rn(vr.luck[S.slot], luck); S.step = 0; }
+            }
         }
         v = c.v;
         const int off1 = __shfl_sync(kFull, v, 26), off2 = __shfl_sync(kFull, v, 27);
@@ -162,6 +226,20 @@ k_rollout(RolloutParams p, const int32_t *__restrict__ Ti, StealResult *__restri
         // Reconverge before the back-edge (see k_selfplay): otherwise every *_sync intrinsic of the walk is guarded by BRA.DIV
         __syncwarp();
     }
+}
+
+template <int kWarps, int kSets>
+__global__ void __launch_bounds__(kWarps * 32, 1)
+k_rollout(RolloutParams p, const int32_t *__restrict__ Ti, StealResult *__restrict__ steal)
+{
+    rollout_loop<kWarps, kSets, false>(p, RolloutVR{0, nullptr, nullptr, nullptr}, Ti, steal);
+}
+
+template <int kWarps, int kSets>
+__global__ void __launch_bounds__(kWarps * 32, 1)
+k_rollout_vr(RolloutParams p, RolloutVR vr, const int32_t *__restrict__ Ti, StealResult *__restrict__ steal)
+{
+    rollout_loop<kWarps, kSets, true>(p, vr, Ti, steal);
 }
 
 // per position: mean and standard error of x_t, float64, each sum in trial order (d * d rounded before it is added: no FMA
@@ -193,6 +271,28 @@ __global__ void k_rollout_reduce(const float *__restrict__ value, const int8_t *
             c[7] += plies[q * trials + t];
         }
         for (int k = 0; k < 8; k++) counts[q * 8 + k] = c[k];
+    }
+}
+
+// per position: mean and standard error of y_t = x_t - luck_t, each sum in trial order exactly as k_rollout_reduce forms them
+__global__ void k_rollout_vr_reduce(const float *__restrict__ value, const double *__restrict__ luck, long long n_pos, int trials,
+                                    double *mean, double *std_err)
+{
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_pos) return;
+    const float *x = value + q * trials;
+    const double *l = luck + q * trials;
+    double sum = 0.0;
+    for (int t = 0; t < trials; t++) sum = __dadd_rn(sum, __dadd_rn((double)x[t], -l[t]));
+    const double m = sum / (double)trials;
+    if (mean) mean[q] = m;
+    if (std_err) {
+        double ss = 0.0;
+        for (int t = 0; t < trials; t++) {
+            const double d = __dadd_rn(__dadd_rn((double)x[t], -l[t]), -m);
+            ss = __dadd_rn(ss, __dmul_rn(d, d));
+        }
+        std_err[q] = trials > 1 ? sqrt(ss / ((double)trials * (double)(trials - 1))) : __longlong_as_double(0x7ff8000000000000ll);
     }
 }
 

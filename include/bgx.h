@@ -230,6 +230,27 @@ int bgx_rollout_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t 
                      double *mean, double *std_err, int64_t *counts,
                      float *trial_value, int8_t *trial_outcome, int32_t *trial_plies);
 
+/* Variance-reduced rollouts (luck-based, as strong backgammon programs do it): bgx_rollout's arguments, play and outputs, bit for
+ * bit, plus the luck of every trial.  For each ply k < min(vr_plies, plies the trial played), with s_k the position before the
+ * roll and p its mover:
+ *   roll value  L_k(a, b) for each of the 21 rolls (a = 1..6, b = 1..a, weight 2 if a != b) is the value bgx_select_moves reports
+ *               for (s_k, p, a, b), or V(s_k, p) as bgx_evaluate gives it when p has no sequence (or only the empty one of a
+ *               blocked double): two-ply's reply value;
+ *   luck        luck_k = L_k(max(d1, d2), min(d1, d2)) - E_k, E_k = sum(weight * L_k) / 36 in that roll order, all float64, E_k not
+ *               rounded to fp32; (d1, d2) is the roll the trial played (the move is still played with the ordered roll);
+ *   trial luck  luck_t = sum of luck_k in ply order (float64); y_t = x_t - luck_t is an unbiased estimate of the same value.
+ * Outputs, any may be NULL: bgx_rollout's seven, then vr_mean[n] and vr_std_err[n], the mean and standard error of y_t by
+ * bgx_rollout's formulas and order, and trial_luck[n][trials].  vr_plies = 0 gives luck 0 and vr_mean = mean.  A VR ply costs
+ * about 21 plies of play.  BGX_E_INVALID for what bgx_rollout refuses and for vr_plies outside [0, BGX_ROLLOUT_MAX_PLIES]. */
+int bgx_rollout_vr(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                   int32_t vr_plies, double *mean, double *std_err, int64_t *counts,
+                   float *trial_value, int8_t *trial_outcome, int32_t *trial_plies,
+                   double *vr_mean, double *vr_std_err, double *trial_luck);
+int bgx_rollout_vr_host(bgx_engine *e, const int8_t *positions, int64_t n, int32_t trials, int32_t max_plies, uint64_t seed, int flags,
+                        int32_t vr_plies, double *mean, double *std_err, int64_t *counts,
+                        float *trial_value, int8_t *trial_outcome, int32_t *trial_plies,
+                        double *vr_mean, double *vr_std_err, double *trial_luck);
+
 /* The same call, asynchronous: copies and kernel are queued on lane `lane`'s own stream
  * (0 <= lane < BGX_ASYNC_LANES) and the call returns at once; bgx_lane_wait(lane) blocks until
  * that lane's outputs are in the host buffers.  Host buffers should be page-locked and must

@@ -8,9 +8,12 @@ Measured, each with CUDA events on device buffers after a warm-up call of the sa
   * the latency of one position x --trials trials;
   * the mean standard error with and without stratification on the same positions and trial counts;
   * plies/s of a quarter of the positions under each warps-per-CTA setting ("rollout_warps").
+With --vr-plies V1,V2,... it measures variance-reduced rollouts (bgx_rollout_vr, DESIGN 7e) instead: for each vr_plies (0 is the
+plain bgx_rollout) one timed full-game call on the same positions and trials, its wall time, plies/s, expected walks/s, mean squared
+standard error, efficiency 1 / (SE^2 x seconds) and the median per-position ratio vr_std_err / std_err.
 The card's name and power limit are read in the same run (nvidia-smi, read-only query).
 
-    python tools/rollout_bench.py [--positions 4096] [--trials 1296] [--out results.json]
+    python tools/rollout_bench.py [--positions 4096] [--trials 1296] [--vr-plies 0,2,8,4096] [--out results.json]
 """
 import argparse
 import json
@@ -57,6 +60,7 @@ def main():
     ap.add_argument("--positions", type=int, default=4096)
     ap.add_argument("--trials", type=int, default=1296)
     ap.add_argument("--slots", type=int, default=65536, help="self-play games of the bgx_selfplay_step comparison")
+    ap.add_argument("--vr-plies", default=None, help="comma-separated vr_plies values: measure variance-reduced rollouts")
     ap.add_argument("--out", default=None, help="also write the result as JSON to this file")
     a = ap.parse_args()
     import torch
@@ -80,6 +84,11 @@ def main():
 
     def run(p, T=0, stratify=True):
         return lambda: eng.rollout(p, a.trials, max_plies=T, stratify=stratify)
+
+    if a.vr_plies is not None:
+        res["vr"] = {v: vr_row(eng, pd, a.trials, int(v)) for v in a.vr_plies.split(",")}
+        finish(eng, res, a.out)
+        return
 
     # the self-play reference: greedy bgx_selfplay_step over a population, plies/s
     eng.selfplay_init(a.slots, first_id=0, id_stride=a.slots, seed=7, first_mover=FIRST_PARITY)
@@ -122,11 +131,38 @@ def main():
         res["warps"][warps] = {"ms": ms, "plies_per_s": int(out["counts"][:, 7].sum().item()) / (ms * 1e-3)}
     eng.set_option("rollout_warps", 20)
     print(f"warps: {json.dumps(res['warps'])}", flush=True)
+    finish(eng, res, a.out)
+
+
+def vr_row(eng, pd, trials, vr):
+    """one timed full-game rollout of every position at vr_plies = vr (0: bgx_rollout), with its standard errors"""
+    import torch
+    ms, out = timed(lambda: eng.rollout(pd, trials, per_trial=True, vr_plies=vr), min_s=0.0)
+    plies = out["trial_plies"].to(torch.int64)
+    n_plies = int(plies.sum().item())
+    se = out["vr_std_err"] if vr else out["std_err"]
+    # a VR ply walks the 21 rolls and the roll played, once less when d1 >= d2 (21 of the 36 ordered rolls)
+    vr_plies_played = int(plies.clamp(max=vr).sum().item())
+    walks = n_plies + (21 - 21 / 36) * vr_plies_played
+    mse = float((se ** 2).mean().item())
+    r = {"ms": ms, "plies": n_plies, "plies_per_s": n_plies / (ms * 1e-3), "vr_plies_played": vr_plies_played,
+         "walks_per_s_expected": walks / (ms * 1e-3), "mean_se": float(se.mean().item()), "mean_se2": mse,
+         "efficiency": 1.0 / (mse * ms * 1e-3)}
+    if vr:
+        live = out["std_err"] > 0                   # a decided position has no variance to reduce
+        r["median_se_ratio"] = float((out["vr_std_err"][live] / out["std_err"][live]).median().item())
+        r["mean_minus_vr_mean_max_sigma"] = float(((out["mean"] - out["vr_mean"]).abs()[live]
+                                                   / (out["std_err"] ** 2 + out["vr_std_err"] ** 2).sqrt()[live]).max().item())
+    print(f"vr_plies={vr}: {json.dumps(r)}", flush=True)
+    return r
+
+
+def finish(eng, res, out):
     eng.close()
     print(json.dumps(res))
-    if a.out:
-        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
-        with open(a.out, "w") as f:
+    if out:
+        os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
+        with open(out, "w") as f:
             json.dump(res, f, indent=1)
 
 
