@@ -77,39 +77,39 @@ struct Mover {
 
     __device__ __forceinline__ Mover(int ln, int pl) : lane(ln), player(pl) { unit = ln < 24 ? (pl ? -1 : 1) : 1; }
 
-    // legal origins of the mover on state v for one die (bgx_core.h legal_origins) from two ballots
-    __device__ __forceinline__ uint32_t legal_here(int v, int die) const
+    // legal origins of the mover on state v for one die (bgx_core.h legal_origins) from two ballots, in code space
+    __device__ __forceinline__ uint32_t legal_here(int v, int die) const { return legal_origins_at<false>(v, die); }
+    // ... in LANE space: bit l = the checker on lane l may move (the bar origin is lane 24 + player).  Points keep their order
+    // (lane = code - 1), and a mover on the bar has the bar as its only origin, so ascending lanes are the reference's order.
+    __device__ __forceinline__ uint32_t legal_lanes(int v, int die) const { return legal_origins_at<true>(v, die); }
+
+    template <bool kLanes>
+    __device__ __forceinline__ uint32_t legal_origins_at(int v, int die) const
     {
-        uint32_t blots;
-        return legal_and_blots<false>(v, die, blots);
-    }
-    // ... and, on request, the enemy blots of v (one bit per LANE: landing there is a hit), from a third ballot
-    template <bool kBlots>
-    __device__ __forceinline__ uint32_t legal_and_blots(int v, int die, uint32_t &blots) const
-    {
+        constexpr int s = kLanes ? 0 : 1;                                 // point lane l is bit l + s
+        constexpr uint32_t points = 0xFFFFFFu << s;
         const int rel = lane < 24 ? v * unit : v;                         // mover-relative count; bar/off lanes as they are
-        if (kBlots) blots = __ballot_sync(kFull, rel == -1);              // (bar / off lanes hold counts >= 0)
         const uint32_t own = __ballot_sync(kFull, rel > 0);
         const uint32_t blk = __ballot_sync(kFull, rel < -1) & 0xFFFFFFu;  // points the mover cannot land on
-        const uint32_t occ = (own & 0xFFFFFFu) << 1, wall = blk << 1;
+        const uint32_t occ = (own & 0xFFFFFFu) << s, wall = blk << s;
         const bool on_bar = (own >> (24 + player)) & 1u;
         if (player == 0) {
-            if (on_bar) return ((wall >> die) & 1u) ? 0u : 1u;
-            uint32_t legal = occ & ((~wall & kPoints) >> die);
-            if (occ != 0 && (occ & kP1Outside) == 0) {
-                legal |= occ & (1u << (25 - die));
+            if (on_bar) return ((wall >> (die - 1 + s)) & 1u) ? 0u : (kLanes ? 1u << 24 : 1u);
+            uint32_t legal = occ & ((~wall & points) >> die);
+            if (occ != 0 && (occ & (kP1Outside >> (1 - s))) == 0) {
+                legal |= occ & (1u << (24 + s - die));
                 const int hi = highest_bit(occ);
-                if (hi + die > 25) legal |= 1u << hi;
+                if (hi + die > 24 + s) legal |= 1u << hi;
             }
             return legal;
         }
-        if (on_bar) return ((wall >> (25 - die)) & 1u) ? 0u : (1u << 25);
-        uint32_t legal = occ & ((~wall & kPoints) << die) & kPoints;
-        if (occ != 0 && (occ & kP2Outside) == 0) {
-            legal |= occ & (1u << die);
-            const uint32_t any = (__ballot_sync(kFull, v != 0) & 0xFFFFFFu) << 1;   // either colour (SURVEY A.3 Q4)
-            const int hi = highest_bit(any & kP2Window);
-            if (hi < die && ((occ >> hi) & 1u)) legal |= 1u << hi;
+        if (on_bar) return ((wall >> (24 + s - die)) & 1u) ? 0u : (1u << 25);
+        uint32_t legal = occ & ((~wall & points) << die) & points;
+        if (occ != 0 && (occ & (kP2Outside >> (1 - s))) == 0) {
+            legal |= occ & (1u << (die - 1 + s));
+            const uint32_t any = (__ballot_sync(kFull, v != 0) & 0xFFFFFFu) << s;   // either colour (SURVEY A.3 Q4)
+            const int hi = highest_bit(any & (kP2Window >> (1 - s)));
+            if (hi < die - 1 + s && ((occ >> hi) & 1u)) legal |= 1u << hi;
         }
         return legal;
     }

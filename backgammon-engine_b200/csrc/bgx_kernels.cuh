@@ -706,7 +706,7 @@ k_select(const int8_t *__restrict__ queries, long long n, float epsilon, uint32_
         player = __shfl_sync(kFull, player, 0); only = __shfl_sync(kFull, only, 0);
         const Choice c = choose_ply_fast<kSets, kExplore>(root, lane, player, d1, d2, ev, cache, explore, u, only ? only : kFull,
                                                           only ? nullptr : &mine);
-        if (only) deliver_child<kWarps>(sm.share, cta_results, vw, only, c, lane);
+        if (only) deliver_child<kWarps>(sm.share, cta_results, vw, c, lane);
         else {
             store_choice(out, q, c, lane, player);
             if (adv.next) store_advanced(adv, q, n, c.v, lane, player);
@@ -862,7 +862,7 @@ k_selfplay(SelfplayParams p, const int32_t *__restrict__ Ti, const float *__rest
                                                               only ? nullptr : &mine, only ? nullptr : zmine,
                                                               only == 0 && S.carry != 0);              // model.py:180-222
             if (only) {
-                deliver_child<kWarps>(sm.share, cta_results, vw, only, c, lane);
+                deliver_child<kWarps>(sm.share, cta_results, vw, c, lane);
                 continue;
             }
             v = c.v;

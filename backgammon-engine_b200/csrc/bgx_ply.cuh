@@ -28,8 +28,9 @@
 //     and every value the walk branches on is provably warp-uniform for ptxas (ballots, REDUX, shuffles from a fixed
 //     lane): otherwise each *_sync intrinsic of the walk is guarded by BRA.DIV (DESIGN 2.1-11; the kernels reconverge
 //     before every back-edge for the same reason).
-//  6. A MOVE IS (origin lane, landing lane, blot bit).  The node's blots are one ballot; the child state is two lane
-//     compares; what stood on the landing point is fetched only where a pre-activation is computed.
+//  6. A MOVE IS (origin lane, landing lane, blot bit).  Origins are lanes throughout the walk (legal masks, twins, the path);
+//     they become the reference's origin codes only when the chosen sequence is packed (finish_choice).  A node's moves are
+//     computed once for all origins; a child is then one shuffle, two lane tests and a few multiply-adds.
 #pragma once
 #include <climits>
 
@@ -154,6 +155,16 @@ struct PlyEvaluator {
     }
     __device__ __forceinline__ float finish(const int4 &zi, int lane) const { return value_of(output_sum(zi, lane)); }
 };
+
+// a row of the table by its 32-bit shared-memory address (the walk's addresses are formed as plain integers: no generic-pointer
+// window arithmetic per row).  volatile: otherwise the loop-invariant rows of a hit are hoisted out of the walk's loops and held
+// in registers (k_select<20,86> then spills)
+__device__ __forceinline__ int4 lds128(uint32_t a)
+{
+    int4 r;
+    asm volatile("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(a));
+    return r;
+}
 
 // The per-warp cache of one ply.  Two kinds of entries share it:
 //   tag 0      an afterstate that was already scored in this ply (the exact-duplicate filter)
@@ -282,10 +293,10 @@ template <int kSets>
 struct PlyWalk : Mover {
     const PlyEvaluator &ev;
     const PlyCache<kSets> &cache;
-    const int4 *Tme;      // this lane's column of the evaluator's table, from the mover's feature block on (child_z)
+    uint32_t Tme;         // shared address of this lane's column of the evaluator's table, from the mover's feature block on (child_z)
     int dieA, dieB;       // die of even / odd depths
-    uint32_t root_only;   // restricts the root's origins (all ones: no restriction)
-    uint32_t twin_root;   // non-doubles, second pass: the root origins of the FIRST pass' first die (0 in the first pass)
+    uint32_t root_only;   // restricts the root's origin lanes (all ones: no restriction)
+    uint32_t twin_root;   // non-doubles, second pass: the root origin lanes of the FIRST pass' first die (0 in the first pass)
     bool nd;              // a pass of a NON-double: walked by the last two levels (2, 3 -> leaves at 4) of the one walk there is,
                           // so that the kernel carries one copy of the per-depth code instead of two (instruction cache)
     int4 zroot;
@@ -295,13 +306,13 @@ struct PlyWalk : Mover {
     float best_key;       // value, negated for PLAYER2 (who minimises): always maximised, strict > keeps the first
     int best_sum;         // the output sum behind it (negated likewise): a sum that does not beat it cannot beat the value
     int best_v;
-    uint32_t best_path;   // origins 5 bits each, length << 20
+    uint32_t best_path;   // origin lanes 5 bits each, length << 20
     int n_seq, n_scored, n_visited;
 
     __device__ __forceinline__ PlyWalk(const PlyEvaluator &e, const PlyCache<kSets> &c, int ln, int pl)
         : Mover(ln, pl), ev(e), cache(c)
     {
-        Tme = e.T4 + ln + (pl ? 4 * 32 : 0);
+        Tme = smem_u32(e.T4 + ln + (pl ? 4 * 32 : 0));
         root_only = kFull;
         twin_root = 0;
         nd = false;
@@ -312,10 +323,12 @@ struct PlyWalk : Mover {
         zstash = nullptr; z_ok = false;
     }
 
-    // What moving one checker does, as a word: bits 0..4 the landing lane | bit 5 a hit | bits 16..23 the row the origin loses |
-    // bits 24..31 the row the landing lane gains.  Rows are rows of Tme = this lane's column of the table shifted to the MOVER's
-    // feature block (row 8 p + k of Tme: "k + 1 checkers of the mover on point p"; the other rows follow from the player by one
-    // multiply-add).  src / dst: the origin and landing lanes (bar 24 + player, borne off 26 + player), sval / dval: what stands there.
+    // What moving one checker does, as a word: bits 0..4 the landing lane | bits 5..12 the row the origin loses | bits 23..30 the
+    // row the landing lane gains | bit 31 a hit.  The fields sit where a child reads them with few instructions: the landing lane
+    // is XOR-compared with the lane in place, the low 13 bits masked to the origin row are that row's offset / 16, the hit is the
+    // sign.  Rows are rows of Tme = this lane's column of the table shifted to the MOVER's feature block (row
+    // 8 p + k of Tme: "k + 1 checkers of the mover on point p"; the other rows follow from the player by one multiply-add).
+    // src / dst: the origin and landing lanes (bar 24 + player, borne off 26 + player), sval / dval: what stands there.
     __device__ __forceinline__ uint32_t move_word(int sval, int dval, int src, int dst) const
     {
         const int n = sval < 0 ? -sval : sval;
@@ -324,7 +337,7 @@ struct PlyWalk : Mover {
         const bool hit = dst < 24 && dval * unit_of_points() == -1;
         int row_dst = dst >= 24 ? kFeatures + 11 * player + dval : 8 * dst + (k < 4 ? k : 4) - 1;   // (198 + 15 player) - 4 player
         if (hit) row_dst = 8 * dst;
-        return (uint32_t)dst | (hit ? 32u : 0u) | ((uint32_t)row_src & 0xFFu) << 16 | (uint32_t)row_dst << 24;
+        return (uint32_t)dst | ((uint32_t)row_src & 0xFFu) << 5 | ((uint32_t)row_dst & 0xFFu) << 23 | (hit ? 1u << 31 : 0u);
     }
     // ... for ALL origins of a node at once: lane l computes the word of "the checker on lane l moves by the node's die" (a garbage
     // word where no legal origin stands); a child then costs one shuffle instead of this arithmetic per child
@@ -335,31 +348,27 @@ struct PlyWalk : Mover {
         if (lane >= 24) dl = player ? 24 - die : die - 1;                // from the bar (game.cpp:89-97)
         return move_word(v, __shfl_sync(kFull, v, dl), lane, dl);
     }
-    // the lane of an origin code
-    __device__ __forceinline__ int origin_lane(int o) const { return o == (player ? 25 : 0) ? 24 + player : o - 1; }
-
     // the child state (game.cpp:624-659): the checker leaves lane sl and lands where the word says
     __device__ __forceinline__ int apply_word(int v, int sl, uint32_t mv) const
     {
-        const int dl = (int)(mv & 31u);
-        const uint32_t hit = (mv >> 5) & 1u;
-        int t = lane == dl ? unit << hit : 0;                // the checker lands, a blot is replaced
+        const int hit = (int)(mv >> 31);
+        int t = v + (lane == 25 - player ? hit : 0);                         // a hit sends the blot to the enemy's bar ...
+        t += ((mv ^ (uint32_t)lane) & 31u) == 0u ? unit + hit * unit : 0;   // ... where the checker lands
         t -= lane == sl ? unit : 0;
-        t += (lane == 25 - player ? 1 : 0) & (int)hit;       // ... and goes to the enemy's bar
-        return v + t;
+        return t;
     }
 
-    // pre-activation of the child reached from zpar by the move mv: 2 rows, 4 after a hit
+    // pre-activation of the child reached from zpar by the move mv: 2 rows, 4 after a hit (a row is 512 bytes)
     __device__ __forceinline__ int4 child_z(const int4 &zpar, uint32_t mv) const
     {
         int4 z = zpar;
-        PlyEvaluator::sub(z, Tme[((mv >> 16) & 0xFFu) * 32]);               // one checker less on the origin (or the bar)
-        if (mv & 32u) {                                                     // a hit
-            const int dst = (int)(mv & 31u);
-            PlyEvaluator::sub(z, Tme[(8 * dst + 4 - 8 * player) * 32]);     // the blot leaves (the enemy's block: +4 / -4) ...
-            PlyEvaluator::add(z, Tme[(195 - 5 * player) * 32]);             // ... for the enemy's bar: (195 - player) - 4 player
+        PlyEvaluator::sub(z, lds128(Tme + ((mv & 0x1FE0u) << 4)));          // one checker less on the origin (or the bar)
+        if ((int)mv < 0) {                                                  // a hit
+            const uint32_t dst = mv & 31u;
+            PlyEvaluator::sub(z, lds128(Tme + (8 * dst + 4 - 8 * player) * 512));   // the blot leaves (the enemy's block: +4 / -4) ...
+            PlyEvaluator::add(z, lds128(Tme + (195 - 5 * player) * 512));           // ... for the enemy's bar: (195 - player) - 4 player
         }
-        PlyEvaluator::add(z, Tme[(mv >> 24) * 32]);                         // one more on the landing point (or borne off)
+        PlyEvaluator::add(z, lds128(Tme + ((mv >> 14) & 0x1FE00u)));         // one more on the landing point (or borne off)
         return z;
     }
 
@@ -406,8 +415,9 @@ struct PlyWalk : Mover {
     // (.., o', o) leads to whenever o' was already playable BEFORE o: in a double when o' is a smaller origin of the parent
     // node, in the second pass of a non-double when o' is a root origin of the first pass.  The reference visits that twin
     // EARLIER (ascending origins; first pass first), it has the same value, and the strict first-index arg-best can never
-    // prefer the later copy: such leaves are counted, not walked.  `legal_par` = all origins of the parent node.
-    // (v, path) = the node; zpar its parent's pre-activation, mv the word of the move that led here (path holds its origin code),
+    // prefer the later copy: such leaves are counted, not walked.  `legal_par` = all origins of the parent node.  (In lane space
+    // "smaller" is "a lower lane": the orders differ only at the bar, and a mover on the bar has no other origin.)
+    // (v, path) = the node; zpar its parent's pre-activation, mv the word of the move that led here (path holds its origin lane),
     // left: that move bore a checker off (kept apart from mv: it steers the walk and has to be provably warp-uniform)
     template <int D>
     __device__ __forceinline__ void visit(int v, const int4 &zpar, uint32_t mv, bool left, uint32_t path, uint32_t legal_par = 0)
@@ -416,7 +426,7 @@ struct PlyWalk : Mover {
         uint32_t legal = 0;
         if constexpr (D < kMax) {
             if (D == 1 && nd) legal = 1u;                    // a non-double pass enters at level 2: level 1 hands the root through
-            else legal = legal_here(v, (D & 1) ? dieB : dieA);
+            else legal = legal_lanes(v, (D & 1) ? dieB : dieA);
             if (D == 0) legal &= root_only;
         }
         uint32_t twins = 0;
@@ -424,7 +434,7 @@ struct PlyWalk : Mover {
             const int die = (D & 1) ? dieB : dieA;
             const int o = (int)((path >> (5 * (D - 1))) & 31u);
             twins = legal & (nd ? twin_root : legal_par & ((1u << o) - 1u));
-            twins &= player ? ~((2u << die) - 1u) : (1u << (25 - die)) - 1u;      // the last move stays on the board ...
+            twins &= player ? ~((1u << die) - 1u) : ((1u << (24 - die)) - 1u) | (1u << 24);   // the last move stays on the board ...
             if (left) twins = 0;                                                 // ... and so did the one before it
         }
         if (legal == 0) {
@@ -453,20 +463,19 @@ struct PlyWalk : Mover {
             if (D != 0 && !(D <= 2 && nd)) z = child_z(zpar, mv);
             const int die = (D & 1) ? dieB : dieA;
             const uint32_t moves = (D == 1 && nd) ? 0u : node_moves(v, die);
+            if (!(D == 1 && nd)) n_visited += __popc(legal);      // the moves applied below
             do {
-                const int oc = lowest_bit(legal);
+                const int sc = lowest_bit(legal);
                 legal &= legal - 1;
                 int child = v;
                 uint32_t mc = 0;
                 bool off = false;
                 if (!(D == 1 && nd)) {
-                    const int sc = origin_lane(oc);
                     mc = __shfl_sync(kFull, moves, sc);
                     child = apply_word(v, sc, mc);
-                    if (D + 1 == kMax - 1) off = (unsigned)(oc + die * unit_of_points() - 1) > 23u;   // (game.cpp:89-97)
-                    n_visited++;
+                    if (D + 1 == kMax - 1) off = sc < 24 && (unsigned)(sc + die * unit_of_points()) > 23u;   // (game.cpp:89-97)
                 }
-                visit<D + 1>(child, z, mc, off, path | ((uint32_t)oc << (5 * D)), legal_all);
+                visit<D + 1>(child, z, mc, off, path | ((uint32_t)sc << (5 * D)), legal_all);
             } while (legal);
             if constexpr (D >= 2) { if (!nd) cache.template store<D>(v, n_seq - entered, lane); }
         }
@@ -523,6 +532,7 @@ struct ShareCtx {
     int giant_min;                       // root origins from which a double is urgent wherever it sits in the queue
 };
 
+// best_path holds origin LANES; the packed moves carry the reference's origin codes (the bar: 0 for PLAYER1, 25 for PLAYER2)
 __device__ __forceinline__ Choice finish_choice(const uint32_t best_path, float best_key, int best_v, int n_seq, int n_scored,
                                                 int n_visited, int root, int player, int d1, int d2, uint32_t best_pass)
 {
@@ -536,7 +546,8 @@ __device__ __forceinline__ Choice finish_choice(const uint32_t best_path, float 
         const int len = (int)(best_path >> 20);
         mv = (uint64_t)len << 40;
         for (int j = 0; j < len; j++) {
-            const int o = (int)((best_path >> (5 * j)) & 31u);
+            const int l = (int)((best_path >> (5 * j)) & 31u);
+            const int o = l >= 24 ? 25 * player : l + 1;
             const int die = ((j & 1) != (int)best_pass) ? d2 : d1;
             mv |= pack_move(o, destination(player, o, die), j);
         }
@@ -546,7 +557,7 @@ __device__ __forceinline__ Choice finish_choice(const uint32_t best_path, float 
     return best;
 }
 
-// root_only: bit mask over the root's origin codes (a helper walks one stolen child); kFull = the whole turn.
+// root_only: bit mask over the root's origin lanes (a helper walks one stolen child); kFull = the whole turn.
 // slot/results: the caller's sharing slot (nullptr: never publish).
 // zstash: this lane's 16 bytes for the pre-activation of the best afterstate (nullptr: none); carry: it holds the
 // pre-activation of `root` as the PREVIOUS mover's walk scored it (same game, one ply earlier): fixed-point sums do not depend
@@ -581,7 +592,7 @@ __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int
     w.dieA = d1; w.dieB = d2;
     w.nd = !dbl;
     if (dbl) {
-        legal = w.legal_here(root, d1) & root_only;
+        legal = w.legal_lanes(root, d1) & root_only;
         if (legal == 0) {
             w.early_leaf(root, 0u);                                      // no move at all: the empty sequence (SURVEY A.3 Q6)
         } else {
@@ -627,15 +638,14 @@ __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int
             }
             if (bit == 0) break;
             oc = lowest_bit(bit);
-            const int sc = w.origin_lane(oc);
-            mroot = __shfl_sync(kFull, root_moves, sc);
-            child = w.apply_word(root, sc, mroot);
+            mroot = __shfl_sync(kFull, root_moves, oc);
+            child = w.apply_word(root, oc, mroot);
             w.n_visited++;
         } else {                                                         // game.cpp:143-188: d1 first, then d2 first
             if (pass == 2) break;
             w.dieA = pass ? d2 : d1;
             w.dieB = pass ? d1 : d2;
-            if (pass) { key1 = w.best_key; w.twin_root = w.legal_here(root, d1); }
+            if (pass) { key1 = w.best_key; w.twin_root = w.legal_lanes(root, d1); }
             pass++;
         }
         w.template visit<1>(child, w.zroot, mroot, false, (uint32_t)oc);
@@ -718,7 +728,7 @@ __device__ __forceinline__ uint32_t take_child(StealShared<kWarps> *sh, int lane
 }
 
 template <int kWarps>
-__device__ __forceinline__ void deliver_child(StealShared<kWarps> *sh, StealResult *cta_results, int vw, uint32_t bit, const Choice &c, int lane)
+__device__ __forceinline__ void deliver_child(StealShared<kWarps> *sh, StealResult *cta_results, int vw, const Choice &c, int lane)
 {
     StealSlot *vs = &sh->slot[vw];
     uint32_t idx = 0;
@@ -728,7 +738,7 @@ __device__ __forceinline__ void deliver_child(StealShared<kWarps> *sh, StealResu
     r->v[lane] = (int8_t)c.v;
     if (lane == 0) {
         r->value = c.value; r->any = c.any ? 1 : 0; r->n_seq = c.n_seq; r->n_scored = c.n_scored;
-        r->n_visited = c.n_visited; r->origin = lowest_bit(bit); r->moves = c.moves;
+        r->n_visited = c.n_visited; r->origin = (int)(c.moves & 31u); r->moves = c.moves;   // the stolen origin's code
     }
     __threadfence_block();
     __syncwarp();

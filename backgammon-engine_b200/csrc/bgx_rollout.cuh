@@ -174,7 +174,7 @@ __device__ __forceinline__ void rollout_loop(RolloutParams p, RolloutVR vr, cons
                                                                                        : zmine),
                                                        only == 0 && !listed && S.carry != 0);
         if (only) {
-            deliver_child<kWarps>(sm.share, cta_results, vw, only, c, lane);
+            deliver_child<kWarps>(sm.share, cta_results, vw, c, lane);
             continue;
         }
         if constexpr (kVR) {
