@@ -28,11 +28,18 @@ constexpr int kFixedBytes = kFixedInts * 4;                       // 118 784
 constexpr int kRowB1 = kFeatures + 30;                            // round(b1 S)
 constexpr int kRowW2 = kFeatures + 31;                            // w2 (fp32 bit patterns)
 constexpr int kRowConst = kFeatures + 32;                         // every float4: {S, -log2(e)/S, b2, Y}
-constexpr int kRowLane = kFeatures + 33;                          // word l (l < 32): the hash multiplier of lane l (PlyCache)
+constexpr int kRowLane = kFeatures + 33;                          // word l (l < 32): the hash multiplier of lane l (PlyCache);
+                                                                  // word 32 + l: the same in PLAYER2's mover frame
 
 // the ply cache's hash multiplier of a lane: odd, and not a polynomial in the lane (moving a checker by the same die from
 // different points must not shift the hash by the same amount)
 __host__ __device__ constexpr uint32_t ply_hash_multiplier(int lane) { return (0x9E3779B1u * (uint32_t)(2 * lane + 1)) ^ (0x85EBCA77u >> (lane & 7)); }
+// ... of a lane of PLAYER2's mover frame (bgx_ply.cuh mover_frame: points negated, 24 <-> 25, 26 <-> 27): a position hashes
+// to the same value in either frame, so the ply cache picks the same sets and victims whoever moves
+__host__ __device__ constexpr uint32_t ply_hash_multiplier_p2(int lane)
+{
+    return lane < 24 ? 0u - ply_hash_multiplier(lane) : ply_hash_multiplier(lane < 28 ? lane ^ 1 : lane);
+}
 
 // status byte (record byte 31) of a self-play slot
 enum { kRunning = 0, kP1Won = 1, kP2Won = 2, kTruncated = 3 };
@@ -78,38 +85,30 @@ struct Mover {
     __device__ __forceinline__ Mover(int ln, int pl) : lane(ln), player(pl) { unit = ln < 24 ? (pl ? -1 : 1) : 1; }
 
     // legal origins of the mover on state v for one die (bgx_core.h legal_origins) from two ballots, in code space
-    __device__ __forceinline__ uint32_t legal_here(int v, int die) const { return legal_origins_at<false>(v, die); }
-    // ... in LANE space: bit l = the checker on lane l may move (the bar origin is lane 24 + player).  Points keep their order
-    // (lane = code - 1), and a mover on the bar has the bar as its only origin, so ascending lanes are the reference's order.
-    __device__ __forceinline__ uint32_t legal_lanes(int v, int die) const { return legal_origins_at<true>(v, die); }
-
-    template <bool kLanes>
-    __device__ __forceinline__ uint32_t legal_origins_at(int v, int die) const
+    __device__ __forceinline__ uint32_t legal_here(int v, int die) const
     {
-        constexpr int s = kLanes ? 0 : 1;                                 // point lane l is bit l + s
-        constexpr uint32_t points = 0xFFFFFFu << s;
         const int rel = lane < 24 ? v * unit : v;                         // mover-relative count; bar/off lanes as they are
         const uint32_t own = __ballot_sync(kFull, rel > 0);
         const uint32_t blk = __ballot_sync(kFull, rel < -1) & 0xFFFFFFu;  // points the mover cannot land on
-        const uint32_t occ = (own & 0xFFFFFFu) << s, wall = blk << s;
+        const uint32_t occ = (own & 0xFFFFFFu) << 1, wall = blk << 1;
         const bool on_bar = (own >> (24 + player)) & 1u;
         if (player == 0) {
-            if (on_bar) return ((wall >> (die - 1 + s)) & 1u) ? 0u : (kLanes ? 1u << 24 : 1u);
-            uint32_t legal = occ & ((~wall & points) >> die);
-            if (occ != 0 && (occ & (kP1Outside >> (1 - s))) == 0) {
-                legal |= occ & (1u << (24 + s - die));
+            if (on_bar) return ((wall >> die) & 1u) ? 0u : 1u;
+            uint32_t legal = occ & ((~wall & kPoints) >> die);
+            if (occ != 0 && (occ & kP1Outside) == 0) {
+                legal |= occ & (1u << (25 - die));
                 const int hi = highest_bit(occ);
-                if (hi + die > 24 + s) legal |= 1u << hi;
+                if (hi + die > 25) legal |= 1u << hi;
             }
             return legal;
         }
-        if (on_bar) return ((wall >> (24 + s - die)) & 1u) ? 0u : (1u << 25);
-        uint32_t legal = occ & ((~wall & points) << die) & points;
-        if (occ != 0 && (occ & (kP2Outside >> (1 - s))) == 0) {
-            legal |= occ & (1u << (die - 1 + s));
-            const uint32_t any = (__ballot_sync(kFull, v != 0) & 0xFFFFFFu) << s;   // either colour (SURVEY A.3 Q4)
-            const int hi = highest_bit(any & (kP2Window >> (1 - s)));
-            if (hi < die - 1 + s && ((occ >> hi) & 1u)) legal |= 1u << hi;
+        if (on_bar) return ((wall >> (25 - die)) & 1u) ? 0u : (1u << 25);
+        uint32_t legal = occ & ((~wall & kPoints) << die) & kPoints;
+        if (occ != 0 && (occ & kP2Outside) == 0) {
+            legal |= occ & (1u << die);
+            const uint32_t any = (__ballot_sync(kFull, v != 0) & 0xFFFFFFu) << 1;   // either colour (SURVEY A.3 Q4)
+            const int hi = highest_bit(any & kP2Window);
+            if (hi < die && ((occ >> hi) & 1u)) legal |= 1u << hi;
         }
         return legal;
     }

@@ -133,7 +133,8 @@ __global__ void k_build_fixed(const float *__restrict__ flat, const float *__res
         const float c[4] = {S, -1.4426950408889634f * aux[1], flat[kTableFloats + 2 * kHidden], aux[3]};
         Ti[idx] = __float_as_int(c[j & 3]);
     } else {                                       // what depends on the lane only: read where needed instead of held (or recomputed) in registers
-        Ti[idx] = j < 32 ? (int32_t)ply_hash_multiplier(j) : 0;       // word l of the row: lane l's multiplier (one bank per lane)
+        // word l of the row: lane l's multiplier (one bank per lane); word 32 + l: the same in PLAYER2's mover frame
+        Ti[idx] = j < 32 ? (int32_t)ply_hash_multiplier(j) : (j < 64 ? (int32_t)ply_hash_multiplier_p2(j - 32) : 0);
     }
 }
 

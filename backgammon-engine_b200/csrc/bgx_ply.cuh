@@ -31,6 +31,8 @@
 //  6. A MOVE IS (origin lane, landing lane, blot bit).  Origins are lanes throughout the walk (legal masks, twins, the path);
 //     they become the reference's origin codes only when the chosen sequence is packed (finish_choice).  A node's moves are
 //     computed once for all origins; a child is then one shuffle, two lane tests and a few multiply-adds.
+//  7. THE MOVER'S FRAME.  A ply converts its root once so that the mover's checkers are positive and its bar / borne-off lanes are
+//     24 / 26 whoever moves (mover_frame), and converts the chosen afterstate back once: a move adds and removes plain ones.
 #pragma once
 #include <climits>
 
@@ -263,10 +265,21 @@ struct PlyCache {
     }
 };
 
+// The greedy walk sees every position in the MOVER'S FRAME (DESIGN 2.1-20): for PLAYER2 the point lanes are negated and the
+// bar lanes (24, 25) and borne-off lanes (26, 27) swap, so the mover's checkers are positive, its bar is lane 24 and its
+// borne-off count lane 26 whoever moves.  Points keep their lanes (ascending lanes stay the reference's origin order for both
+// players); the direction of travel and the bear-off rules stay per player.  The map is its own inverse.
+__device__ __forceinline__ int mover_frame(int v, int lane, int player)
+{
+    const int w = __shfl_sync(kFull, v, player && (unsigned)(lane - 24) < 4u ? lane ^ 1 : lane);
+    return player && lane < 24 ? -w : w;
+}
+
 // A sequence that ends before the dice are used up (no legal move left) is the rare kind of leaf.  Its
 // afterstate is scored FROM SCRATCH by this out-of-line routine - the fixed-point z of a position does not
 // depend on how it is computed - so the fully inlined walk carries the leaf code only at its last level
-// (the kernel's code has to stay close to the 32 KB instruction cache).  Returns the output sum, kSeenBefore if scored before.
+// (the kernel's code has to stay close to the 32 KB instruction cache).  v is in the mover's frame.  Returns the output sum,
+// kSeenBefore if scored before.
 constexpr int kSeenBefore = INT_MIN;
 template <int kSets>
 __device__ __noinline__ int score_early_leaf(uint8_t *col, uint32_t meta, const uint32_t *kmul, const int4 *T4, int v, int lane, int player)
@@ -278,7 +291,7 @@ __device__ __noinline__ int score_early_leaf(uint8_t *col, uint32_t meta, const 
     cache.template write<0>(pr, v, 0, lane);
     PlyEvaluator e;
     e.T4 = T4;
-    return e.output_sum(e.preactivation(v, lane, player), lane);
+    return e.output_sum(e.preactivation(mover_frame(v, lane, player), lane, player), lane);
 }
 
 // ---- the walk ----------------------------------------------------------------------------
@@ -289,10 +302,14 @@ __device__ __noinline__ int score_early_leaf(uint8_t *col, uint32_t meta, const 
 // shuffle for the landing point, three predicated adds) and probed in the cache; the rows its
 // move changes in the network input, its pre-activation and its value are computed only for
 // afterstates that were not scored yet in this ply and for interior nodes.
+// Every state of the walk is in the mover's frame (mover_frame): the mover's checkers count +1 wherever they stand, so a move
+// adds and removes plain ones and the player is left only in the direction of travel, the bear-off rules, the table rows and
+// the value's sign, all uniform per ply.
 template <int kSets>
-struct PlyWalk : Mover {
+struct PlyWalk {
     const PlyEvaluator &ev;
     const PlyCache<kSets> &cache;
+    int lane, player;
     uint32_t Tme;         // shared address of this lane's column of the evaluator's table, from the mover's feature block on (child_z)
     int dieA, dieB;       // die of even / odd depths
     uint32_t root_only;   // restricts the root's origin lanes (all ones: no restriction)
@@ -310,7 +327,7 @@ struct PlyWalk : Mover {
     int n_seq, n_scored, n_visited;
 
     __device__ __forceinline__ PlyWalk(const PlyEvaluator &e, const PlyCache<kSets> &c, int ln, int pl)
-        : Mover(ln, pl), ev(e), cache(c)
+        : ev(e), cache(c), lane(ln), player(pl)
     {
         Tme = smem_u32(e.T4 + ln + (pl ? 4 * 32 : 0));
         root_only = kFull;
@@ -328,14 +345,12 @@ struct PlyWalk : Mover {
     // is XOR-compared with the lane in place, the low 13 bits masked to the origin row are that row's offset / 16, the hit is the
     // sign.  Rows are rows of Tme = this lane's column of the table shifted to the MOVER's feature block (row
     // 8 p + k of Tme: "k + 1 checkers of the mover on point p"; the other rows follow from the player by one multiply-add).
-    // src / dst: the origin and landing lanes (bar 24 + player, borne off 26 + player), sval / dval: what stands there.
+    // src / dst: the origin and landing lanes (bar 24, borne off 26), sval / dval: what stands there.
     __device__ __forceinline__ uint32_t move_word(int sval, int dval, int src, int dst) const
     {
-        const int n = sval < 0 ? -sval : sval;
-        const int row_src = src >= 24 ? 194 - 3 * player : 8 * src + (n < 4 ? n : 4) - 1;           // (194 + player) - 4 player
-        const int k = (dval < 0 ? -dval : dval) + 1;
-        const bool hit = dst < 24 && dval * unit_of_points() == -1;
-        int row_dst = dst >= 24 ? kFeatures + 11 * player + dval : 8 * dst + (k < 4 ? k : 4) - 1;   // (198 + 15 player) - 4 player
+        const int row_src = src >= 24 ? 194 - 3 * player : 8 * src + (sval < 4 ? sval : 4) - 1;      // (194 + player) - 4 player
+        const bool hit = dval == -1;                                     // (only points hold the enemy's checkers, negative)
+        int row_dst = dst >= 24 ? kFeatures + 11 * player + dval : 8 * dst + (dval < 3 ? dval : 3);  // (198 + 15 player) - 4 player
         if (hit) row_dst = 8 * dst;
         return (uint32_t)dst | ((uint32_t)row_src & 0xFFu) << 5 | ((uint32_t)row_dst & 0xFFu) << 23 | (hit ? 1u << 31 : 0u);
     }
@@ -343,8 +358,8 @@ struct PlyWalk : Mover {
     // word where no legal origin stands); a child then costs one shuffle instead of this arithmetic per child
     __device__ __forceinline__ uint32_t node_moves(int v, int die) const
     {
-        const int d = lane + die * unit_of_points();                     // from a point: the landing point, or off the board
-        int dl = (unsigned)d > 23u ? 26 + player : d;
+        const int d = lane + die * dir();                                // from a point: the landing point, or off the board
+        int dl = (unsigned)d > 23u ? 26 : d;
         if (lane >= 24) dl = player ? 24 - die : die - 1;                // from the bar (game.cpp:89-97)
         return move_word(v, __shfl_sync(kFull, v, dl), lane, dl);
     }
@@ -352,10 +367,39 @@ struct PlyWalk : Mover {
     __device__ __forceinline__ int apply_word(int v, int sl, uint32_t mv) const
     {
         const int hit = (int)(mv >> 31);
-        int t = v + (lane == 25 - player ? hit : 0);                         // a hit sends the blot to the enemy's bar ...
-        t += ((mv ^ (uint32_t)lane) & 31u) == 0u ? unit + hit * unit : 0;   // ... where the checker lands
-        t -= lane == sl ? unit : 0;
+        int t = v + (lane == 25 ? hit : 0);                                  // a hit sends the blot to the enemy's bar ...
+        t += ((mv ^ (uint32_t)lane) & 31u) == 0u ? 1 + hit : 0;              // ... where the checker lands
+        t -= lane == sl ? 1 : 0;
         return t;
+    }
+    __device__ __forceinline__ int dir() const { return player ? -1 : 1; }   // direction of travel on the point lanes
+
+    // legal origin lanes of the mover for one die (bgx_core.h legal_origins in the mover's frame): bit l = the checker on lane l
+    // may move, the bar is lane 24.  Points keep their order (lane = code - 1), and a mover on the bar has the bar as its only
+    // origin, so ascending lanes are the reference's order.
+    __device__ __forceinline__ uint32_t legal_lanes(int v, int die) const
+    {
+        const uint32_t own = __ballot_sync(kFull, v > 0);
+        const uint32_t wall = __ballot_sync(kFull, v < -1) & 0xFFFFFFu;    // points the mover cannot land on
+        const uint32_t occ = own & 0xFFFFFFu;
+        if ((own >> 24) & 1u) return ((wall >> (player ? 24 - die : die - 1)) & 1u) ? 0u : 1u << 24;
+        if (player == 0) {
+            uint32_t legal = occ & ((~wall & 0xFFFFFFu) >> die);
+            if (occ != 0 && (occ & (kP1Outside >> 1)) == 0) {
+                legal |= occ & (1u << (24 - die));
+                const int hi = highest_bit(occ);
+                if (hi + die > 24) legal |= 1u << hi;
+            }
+            return legal;
+        }
+        uint32_t legal = occ & ((~wall & 0xFFFFFFu) << die);
+        if (occ != 0 && (occ & (kP2Outside >> 1)) == 0) {
+            legal |= occ & (1u << (die - 1));
+            const uint32_t any = __ballot_sync(kFull, v != 0) & 0xFFFFFFu;   // either colour (SURVEY A.3 Q4)
+            const int hi = highest_bit(any & (kP2Window >> 1));
+            if (hi < die - 1 && ((occ >> hi) & 1u)) legal |= 1u << hi;
+        }
+        return legal;
     }
 
     // pre-activation of the child reached from zpar by the move mv: 2 rows, 4 after a hit (a row is 512 bytes)
@@ -473,7 +517,7 @@ struct PlyWalk : Mover {
                 if (!(D == 1 && nd)) {
                     mc = __shfl_sync(kFull, moves, sc);
                     child = apply_word(v, sc, mc);
-                    if (D + 1 == kMax - 1) off = sc < 24 && (unsigned)(sc + die * unit_of_points()) > 23u;   // (game.cpp:89-97)
+                    if (D + 1 == kMax - 1) off = sc < 24 && (unsigned)(sc + die * dir()) > 23u;  // (game.cpp:89-97)
                 }
                 visit<D + 1>(child, z, mc, off, path | ((uint32_t)sc << (5 * D)), legal_all);
             } while (legal);
@@ -561,7 +605,9 @@ __device__ __forceinline__ Choice finish_choice(const uint32_t best_path, float 
 // slot/results: the caller's sharing slot (nullptr: never publish).
 // zstash: this lane's 16 bytes for the pre-activation of the best afterstate (nullptr: none); carry: it holds the
 // pre-activation of `root` as the PREVIOUS mover's walk scored it (same game, one ply earlier): fixed-point sums do not depend
-// on how they were formed, so flipping the turn flag gives exactly what preactivation() would compute
+// on how they were formed, so flipping the turn flag gives exactly what preactivation() would compute.
+// root and the returned Choice are in the real frame; the walk runs in the mover's (mover_frame: one conversion each way per
+// ply).  A published double's root stays in the real frame: a helper's greedy_ply converts it and delivers in the real frame.
 template <int kSets>
 __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int d1, int d2, const PlyEvaluator &ev,
                                              PlyCache<kSets> &cache, uint32_t root_only = kFull, const ShareCtx *share = nullptr,
@@ -570,7 +616,10 @@ __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int
     StealSlot *slot = share ? share->slot : nullptr;
     StealResult *results = share ? share->results : nullptr;
     cache.next_ply(lane);
-    PlyWalk<kSets> w(ev, cache, lane, player);
+    PlyCache<kSets> fcache = cache;
+    if (player) fcache.kmul += 32;                                       // the hash multipliers of PLAYER2's frame (kRowLane)
+    const int froot = mover_frame(root, lane, player);
+    PlyWalk<kSets> w(ev, fcache, lane, player);
     w.root_only = root_only;
     if (carry) {
         int4 z = *zstash;
@@ -592,9 +641,9 @@ __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int
     w.dieA = d1; w.dieB = d2;
     w.nd = !dbl;
     if (dbl) {
-        legal = w.legal_lanes(root, d1) & root_only;
+        legal = w.legal_lanes(froot, d1) & root_only;
         if (legal == 0) {
-            w.early_leaf(root, 0u);                                      // no move at all: the empty sequence (SURVEY A.3 Q6)
+            w.early_leaf(froot, 0u);                                     // no move at all: the empty sequence (SURVEY A.3 Q6)
         } else {
             shared = slot != nullptr && __popc(legal) >= kStealMinChildren;
             if (shared) {                                                // publish the root's origins
@@ -614,9 +663,9 @@ __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int
             }
         }
     }
-    const uint32_t root_moves = dbl ? w.node_moves(root, d1) : 0u;
+    const uint32_t root_moves = dbl ? w.node_moves(froot, d1) : 0u;
     for (;;) {
-        int child = root, oc = 0;
+        int child = froot, oc = 0;
         uint32_t mroot = 0;
         if (dbl) {
             uint32_t bit = 0;
@@ -639,13 +688,13 @@ __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int
             if (bit == 0) break;
             oc = lowest_bit(bit);
             mroot = __shfl_sync(kFull, root_moves, oc);
-            child = w.apply_word(root, oc, mroot);
+            child = w.apply_word(froot, oc, mroot);
             w.n_visited++;
         } else {                                                         // game.cpp:143-188: d1 first, then d2 first
             if (pass == 2) break;
             w.dieA = pass ? d2 : d1;
             w.dieB = pass ? d1 : d2;
-            if (pass) { key1 = w.best_key; w.twin_root = w.legal_lanes(root, d1); }
+            if (pass) { key1 = w.best_key; w.twin_root = w.legal_lanes(froot, d1); }
             pass++;
         }
         w.template visit<1>(child, w.zroot, mroot, false, (uint32_t)oc);
@@ -657,7 +706,7 @@ __device__ __forceinline__ Choice greedy_ply(int root, int lane, int player, int
         // levels 2, 3 wrote the origins at bits 10.. and counted the two levels above into the length
         w.best_path = ((w.best_path & 0xFFFFFu) >> 10) | (((w.best_path >> 20) - 2u) << 20);
     }
-    Choice best = finish_choice(w.best_path, w.best_key, w.best_v, w.n_seq, w.n_scored, w.n_visited, root, player, d1, d2, best_pass);
+    Choice best = finish_choice(w.best_path, w.best_key, mover_frame(w.best_v, lane, player), w.n_seq, w.n_scored, w.n_visited, root, player, d1, d2, best_pass);
     best.z_ok = best.any && w.z_ok;
     if (shared) {
         // wait for the helpers, then merge their sub-trees: better value, then lower root origin
